@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Throughput benchmark of the batched FOOTSIES frame update (BASELINE.json metric: env-frames/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--envs-per-gpu E]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--envs-per-gpu E] [--dump-outputs DIR]
 
 One "step" = one FootsiesEnv.step over every env of the rank (frame-skip 1: one BattleCore fight frame per
 env).  Workload (config D of SURVEY.md §8, weak-scaled so that each GPU's working set exceeds the 126 MB L2):
@@ -58,7 +58,30 @@ def parse_args():
                          "(one horizon = one bench step), weak scaling, one stats all-reduce at the end")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (rank 0, a fixed seeded sample "
+                         "of the envs) as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+def dump_outputs(out_dir, n, sample, arrays):
+    """Writes each device tensor of `arrays` ({name: (tensor, env axis)}) at a fixed, seeded sample of `sample` of the
+    N envs as float32 (float64 for integers wider than 16 bits, which float32 may not hold exactly), plus the sampled
+    env indices.  The caller picks `sample` so that the whole dump stays under 64 MB."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, sample), replace=False))
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    for name, (t, axis) in arrays.items():
+        a = t.index_select(axis, torch.from_numpy(idx).to(t.device)).cpu().numpy()
+        wide = a.dtype.kind in "iu" and a.dtype.itemsize > 2
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64 if wide else np.float32))
 
 
 def measured_traffic(bytes_per_env_alg, n):
@@ -176,7 +199,6 @@ def cpu_throughput(kind, n_envs, threads, seconds=None, steps=None, warmup=3, se
 
 
 REF_STEP_ENV_STEPS = 256
-REF_MAX_SECONDS = 30.0
 REF_SAMPLE_ENVS = {"reference": 4096, "port": 32768}     # a transliterated game object graph is ~0.6 MB per battle
 
 
@@ -198,9 +220,8 @@ def run_reference(args, rank, world):
         return
     threads = os.cpu_count() or 1
     # one `step` of this arm = REF_STEP_ENV_STEPS consecutive env-steps of the 4096-battle sample (~1 M env-frames: a few
-    # tenths of a second on the box's cores), so that the driver's `--steps 20` times seconds of CPU work
-    # (bounded: at most REF_MAX_SECONDS, whatever --steps says; the line reports the steps that were timed)
-    base, dt, done = cpu_baseline_entry("reference", threads, steps=args.steps, seconds=REF_MAX_SECONDS, warmup=min(args.warmup, 3),
+    # tenths of a second on a many-core host), so that `--steps 20` times seconds of CPU work
+    base, dt, done = cpu_baseline_entry("reference", threads, steps=args.steps, warmup=min(args.warmup, 3),
                                         inner=REF_STEP_ENV_STEPS)
     port, _, _ = cpu_baseline_entry("port", threads, seconds=3.0)
     value = base["value"]
@@ -237,7 +258,7 @@ def run_rollout(args, rank, world, dev, dist):
     from footsies_gym_b200 import FootsiesEnv
     from footsies_gym_b200.rollout import MLPPolicy, RolloutCollector
     n, horizon = 16384, 128
-    steps = min(args.steps, 200)
+    steps = args.steps
     env = FootsiesEnv(num_envs=n, device=dev, opponent=None, seed=0, first_env_index=rank * n)
     torch.manual_seed(0)
     col = RolloutCollector(env, MLPPolicy(64).to(dev), horizon=horizon, use_cuda_graph=True, seed=rank)
@@ -252,9 +273,12 @@ def run_rollout(args, rank, world, dev, dist):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        col.collect()
+        out = col.collect()
     e1.record()
     torch.cuda.synchronize(dev)
+    if args.dump_outputs and rank == 0:
+        # obs [horizon, N, 8], actions / logp / rewards / dones [horizon, N], last_obs [N, 8]: ~6 KB per env
+        dump_outputs(args.dump_outputs, n, 4096, {k: (v, 0 if k == "last_obs" else 1) for k, v in out.items()})
     if world > 1:
         dist.barrier()
     t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
@@ -293,7 +317,7 @@ def main():
     import numpy as np
     import torch
     import torch.distributed as dist
-    from footsies_gym_b200 import FootsiesEnv
+    from footsies_gym_b200 import FootsiesEnv, _capi
 
     if not torch.cuda.is_available():
         raise SystemExit("bench.py --impl b200 needs a CUDA device; there is no CPU fallback")
@@ -336,55 +360,56 @@ def main():
             dist.barrier()
         torch.cuda.synchronize(dev)
 
-    # how many blocks of `steps` launches: at least 25, and enough for ~0.6 s so that nvidia-smi can sample the clocks
-    # DURING the timed region (50 ms period); every rank uses the same count
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    ev0.record()
-    for i in range(args.steps):
-        device_step(i)
-    ev1.record()
-    torch.cuda.synchronize(dev)
-    est_block_ms = max(ev0.elapsed_time(ev1), 1e-3)
-    blocks_t = torch.tensor([max(25, min(2000, int(600.0 / est_block_ms) + 1))], dtype=torch.int64, device=dev)
-    if world > 1:
-        dist.all_reduce(blocks_t, op=dist.ReduceOp.MAX)
-    blocks = int(blocks_t.item())
-
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
         time.sleep(0.25)
 
-    # ---------------- timed region: `blocks` x K device-resident steps, back to back; the MEDIAN block is reported ------------
-    frames_before = env.episode_stats()["env_frames"]
-    launches_before = env.launch_count()
+    # ---------------- timed region: exactly `steps` device-resident steps, back to back ----------------
+    # an event after every block of `block` steps gives the spread; the value is the whole window
+    block = max(1, args.steps // 25)
     barrier()
-    events = [torch.cuda.Event(enable_timing=True) for _ in range(blocks + 1)]
+    # a few untimed lead-in steps keep the GPU busy while the window opens, so that a short window does not time the
+    # idle GPU's start-up; the frame counter is snapshotted in stream order where the window begins
+    for i in range(4):
+        device_step(i)
+    env_frames = _capi.STAT_NAMES.index("env_frames")
+    frames_before = env.stats[env_frames].clone()
+    launches_before = env.launch_count()
+    events, marks = [torch.cuda.Event(enable_timing=True)], [0]
     wall0 = time.time()
     events[0].record()
-    for b in range(blocks):
-        for i in range(args.steps):
-            device_step(b * args.steps + i)
-        events[b + 1].record()
+    for i in range(args.steps):
+        device_step(i)
+        if (i + 1) % block == 0 or i + 1 == args.steps:
+            events.append(torch.cuda.Event(enable_timing=True))
+            events[-1].record()
+            marks.append(i + 1)
     barrier()
     wall1 = time.time()
-    block_ms = sorted(events[b].elapsed_time(events[b + 1]) for b in range(blocks))
-    ms_local = block_ms[len(block_ms) // 2]
-    frames_local = (env.episode_stats()["env_frames"] - frames_before) / blocks      # per block (steady state)
+    if args.dump_outputs and rank == 0:
+        # what step_bound() returned for the last timed step: obs [N, 8], reward, terminated, truncated, info frame /
+        # actions / hitstun (info's observation keys are views of obs); ~76 bytes per env
+        dump_outputs(args.dump_outputs, n, 1 << 18,
+                     {"obs": (env.obs, 0), "reward": (env.reward, 0), "terminated": (env.terminated, 0),
+                      "truncated": (env.truncated, 0), "info_frame": (env.info_frame, 0), "info_misc": (env.info_misc, 0)})
+    ms_local = events[0].elapsed_time(events[-1])
+    per_step_ms = sorted(events[j].elapsed_time(events[j + 1]) / (marks[j + 1] - marks[j]) for j in range(len(events) - 1))
+    frames_local = int((env.stats[env_frames] - frames_before).item())
     launches = env.launch_count() - launches_before
 
     clocks = None
     if rank == 0:
         clocks = sampler.summary(wall0, wall1) or {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
-        clocks["sampled"] = "nvidia-smi -lms 50 during the %d timed blocks (%.2f s)" % (blocks, wall1 - wall0)
+        clocks["sampled"] = "nvidia-smi -lms 50 during the %d timed steps (%.2f s)" % (args.steps, wall1 - wall0)
         sampler.stop()
 
-    t = torch.tensor([ms_local, -block_ms[0], block_ms[-1]], dtype=torch.float64, device=dev)
+    t = torch.tensor([ms_local, -per_step_ms[0], per_step_ms[-1]], dtype=torch.float64, device=dev)
     f = torch.tensor([frames_local], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dist.all_reduce(f, op=dist.ReduceOp.SUM)
-    ms_total, ms_block_min, ms_block_max = float(t[0].item()), -float(t[1].item()), float(t[2].item())
+    ms_total, ms_step_min, ms_step_max = float(t[0].item()), -float(t[1].item()), float(t[2].item())
     frames_total = float(f.item())
     value = frames_total / (ms_total * 1e-3)
 
@@ -590,16 +615,16 @@ def main():
     if rank == 0:
         peak, peak_src = measured_peaks()
         bytes_per_env = env.algorithmic_bytes_per_env_step
-        ms_per_launch = ms_total / max(args.steps, 1)        # median block / launches per block
+        ms_per_launch = ms_total / args.steps
         achieved = bytes_per_env * n / (ms_per_launch * 1e-3) / 1e9
         traffic, traffic_src = measured_traffic(bytes_per_env, n)
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
-            "warmup": max(args.warmup, 3), "ms_per_step": ms_per_launch, "blocks": blocks,
-            "ms_per_step_min": ms_block_min / max(args.steps, 1), "ms_per_step_max": ms_block_max / max(args.steps, 1),
-            "timing": "the block of `steps` launches is run `blocks` times back to back after the burn-in; value and "
-                      "ms_per_step are the MEDIAN block (CUDA events on the launching stream, max over ranks); "
-                      "min / max are the fastest / slowest block",
+            "warmup": max(args.warmup, 3), "ms_per_step": ms_per_launch,
+            "ms_per_step_min": ms_step_min, "ms_per_step_max": ms_step_max,
+            "timing": "`steps` launches back to back after the burn-in and warm-up; value and ms_per_step are the whole "
+                      "window (CUDA events on the launching stream, max over ranks); min / max are the fastest / slowest "
+                      "of up to 25 equal blocks of the window, per step",
             "higher_is_better": True,
             "scaling": "strong" if args.total_envs > 0 else "weak", "vs_baseline": None, "dtype": "int32+fp32",
             "data": "synthetic",
