@@ -6,8 +6,10 @@
 
 Rollouts come from footsies_gym_b200.rollout.RolloutCollector: the fused policy kernel samples actions from the
 observation tensor the step kernel wrote, the step kernel writes the next observation / reward / done flag straight
-into the rollout buffers, one launch per horizon (fg_rollout_mlp keeps the battles in registers for all 128 steps).  The update is ordinary torch (clipped PPO with GAE, a
-separate value MLP); the policy's parameters are updated in place, so the next rollout reads the new weights.
+into the rollout buffers, one launch per horizon (fg_rollout_mlp keeps the battles in registers for all 128 steps).  The
+collector also evaluates the value MLP over every observation of the horizon (fg_value_mlp, one launch) and computes GAE
+advantages and returns (fg_gae, one launch).  The update is ordinary torch (clipped PPO); the policy's and the value
+network's parameters are updated in place, so the next rollout reads the new weights.
 Prints the win rate against the bot per iteration (from the kernel's own episode statistics).
 With --self-play the training rollouts are played against the same network on the mirrored observation (still one
 launch per horizon) and the win rate against the in-game bot comes from a separate evaluation rollout per iteration.
@@ -23,7 +25,7 @@ import torch
 import torch.distributed as dist
 
 from footsies_gym_b200.distributed import env_rank_world, make_sharded_env
-from footsies_gym_b200.rollout import MLPPolicy, RolloutCollector
+from footsies_gym_b200.rollout import MLPPolicy, MLPValue, RolloutCollector
 
 
 def main():
@@ -51,15 +53,15 @@ def main():
 
     env = make_sharded_env(a.envs * world, frame_skip=a.frame_skip, seed=0, opponent="self_play" if a.self_play else None)
     policy = MLPPolicy(64).to(dev)
-    value = torch.nn.Sequential(torch.nn.Linear(8, 64), torch.nn.Tanh(), torch.nn.Linear(64, 64), torch.nn.Tanh(),
-                                torch.nn.Linear(64, 1)).to(dev)
+    value = MLPValue(64).to(dev)
     params = list(policy.parameters()) + list(value.parameters())
     if world > 1:
         for p in params:
             dist.broadcast(p.data, 0)
     opt = torch.optim.Adam(params, lr=a.lr)
     col = RolloutCollector(env, policy, horizon=a.horizon, use_cuda_graph=True, seed=rank,
-                           opponent_policy=policy if a.self_play else None, mirror_opponent=a.self_play)
+                           opponent_policy=policy if a.self_play else None, mirror_opponent=a.self_play,
+                           value=value, gamma=a.gamma, gae_lambda=a.lam)
     eval_env = eval_col = None
     if a.self_play:                       # the yardstick stays the in-game bot
         eval_env = make_sharded_env(a.envs * world, frame_skip=a.frame_skip, seed=1)
@@ -74,19 +76,12 @@ def main():
         torch.cuda.synchronize(dev)
         t1 = time.perf_counter()
         obs, act, logp_old = out["obs"], out["actions"].long(), out["logp"]
-        rew, done = out["rewards"], out["dones"].float()
+        rew = out["rewards"]
+        # GAE came with the rollout: an env that terminated at step t restarts by itself (the step after is the reset,
+        # reward 0), so the bootstrap is cut at the terminal step
+        ret = out["returns"]
         with torch.no_grad():
-            v = value(torch.cat([obs, out["last_obs"][None]], 0) * policy.scale).squeeze(-1)      # [h + 1, n]
-            # an env that terminated at step t restarts by itself: the step after is the reset (reward 0); cut the
-            # bootstrap at the terminal step
-            adv = torch.zeros_like(rew)
-            last = torch.zeros(n, device=dev)
-            for t in range(h - 1, -1, -1):
-                nonterm = 1.0 - done[t]
-                delta = rew[t] + a.gamma * v[t + 1] * nonterm - v[t]
-                last = delta + a.gamma * a.lam * nonterm * last
-                adv[t] = last
-            ret = adv + v[:h]
+            adv = out["advantages"]
             adv = (adv - adv.mean()) / (adv.std() + 1e-8)
         flat = lambda x: x.reshape(h * n, *x.shape[2:])     # noqa: E731
         fo, fa, fl, fadv, fret = flat(obs), flat(act), flat(logp_old), flat(adv), flat(ret)
@@ -98,7 +93,7 @@ def main():
                 lp = lp_all.gather(1, fa[mb, None]).squeeze(1)
                 ratio = (lp - fl[mb]).exp()
                 pg = -torch.min(ratio * fadv[mb], ratio.clamp(1 - a.clip, 1 + a.clip) * fadv[mb]).mean()
-                vl = 0.5 * (value(fo[mb] * policy.scale).squeeze(-1) - fret[mb]).pow(2).mean()
+                vl = 0.5 * (value(fo[mb]) - fret[mb]).pow(2).mean()
                 ent = -(lp_all.exp() * lp_all).sum(-1).mean()
                 loss = pg + 0.5 * vl - a.entropy * ent
                 opt.zero_grad(set_to_none=True)

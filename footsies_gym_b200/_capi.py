@@ -118,7 +118,7 @@ EXPORTS = ["fg_abi_version", "fg_last_error", "fg_algorithmic_bytes_per_env_step
            "fg_reset_host_compact", "fg_packed_reward_table", "fg_step_host_packed", "fg_reset_host_packed", "fg_host_alloc",
            "fg_host_free", "fg_delay_ring_step", "fg_get_state",
            "fg_set_state", "fg_read_stats", "fg_launch_count", "fg_policy_mlp_sample", "fg_policy_mlp_sample_p2", "fg_policy_last_error",
-           "fg_rollout_mlp"]
+           "fg_rollout_mlp", "fg_value_mlp", "fg_gae"]
 
 
 def load(build_if_missing=True):
@@ -187,6 +187,10 @@ def load(build_if_missing=True):
     L.fg_policy_last_error.restype = C.c_char_p
     L.fg_rollout_mlp.restype = i32
     L.fg_rollout_mlp.argtypes = [vp, C.POINTER(FgRolloutBuffers), vp]
+    L.fg_value_mlp.restype = i32
+    L.fg_value_mlp.argtypes = [vp] * 8 + [i32, i64, vp, vp]
+    L.fg_gae.restype = i32
+    L.fg_gae.argtypes = [vp, vp, vp, i32, i32, C.c_float, C.c_float, vp, vp, vp]
     if L.fg_abi_version() != 2:
         raise FootsiesLibraryError("libfootsies_b200.so ABI version mismatch")
     _lib = L

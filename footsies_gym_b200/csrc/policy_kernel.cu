@@ -8,6 +8,8 @@
 // battles; policy_mlp.cuh); the sampled action is written as the uint8 input bitmask the step kernel is bound to, next
 // to its log-probability, and (optionally) the observation row is copied into the rollout buffer on the way.
 // The per-step path for configurations the whole-horizon kernel (rollout_kernel.cu) does not cover (self-play, masks).
+// Also the critic side of an actor-critic rollout: the value network on the same tensor-core path (fg_value_mlp) and GAE
+// advantages / returns (fg_gae).
 #include "device_once.h"
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -121,6 +123,81 @@ __global__ void __launch_bounds__(32 * kMmaWarps) policy_mma_sample_kernel(const
     }
 }
 
+// Value network V(obs * scale) = Linear(H, 1)(tanh(Linear(H, H)(tanh(Linear(8, H)(obs * scale))))) over `rows` observation
+// rows -- the critic of an actor-critic rollout, over all (horizon + 1) x N rows of a rollout buffer in one launch.  It is
+// the policy's forward pass (policy_mma_logits) with W3 staged as ONE real output row: the value is logit column 0.  Same
+// shape as policy_mma_sample_kernel: persistent grid, weights staged once per CTA, a warp evaluates 32 rows at a time.
+template <int H>
+__global__ void __launch_bounds__(32 * kMmaWarps) value_mma_kernel(const float *__restrict__ obs, const PolicyWeights w,
+                                                                   long long rows, float *__restrict__ values) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float *sm = reinterpret_cast<float *>(smem_raw);
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    float *obs_w = reinterpret_cast<float *>(smem_raw + PolicyMmaKernelSmem<H>::kObs) + warp * 256;
+    float *lg_w = reinterpret_cast<float *>(smem_raw + PolicyMmaKernelSmem<H>::kLogits) + warp * 256;
+    policy_mma_stage<H, 1>(sm, w, tid, 32 * kMmaWarps);
+    __syncthreads();
+    for (long long base = ((long long)blockIdx.x * kMmaWarps + warp) * 32; base < rows; base += (long long)gridDim.x * kMmaWarps * 32) {
+        const long long row = base + lane;
+        const bool valid = row < rows;
+        const float4 a = valid ? reinterpret_cast<const float4 *>(obs)[2 * row] : make_float4(0, 0, 0, 0);
+        const float4 b = valid ? reinterpret_cast<const float4 *>(obs)[2 * row + 1] : make_float4(0, 0, 0, 0);
+        __syncwarp();                                           // the previous group's fragment loads are done
+        reinterpret_cast<float4 *>(obs_w)[2 * lane] = a;
+        reinterpret_cast<float4 *>(obs_w)[2 * lane + 1] = b;
+        __syncwarp();
+        policy_mma_logits<H, 2, false>(sm, obs_w, lg_w, lane);
+        if (valid) values[row] = lg_w[8 * lane];
+    }
+}
+
+// GAE(gamma, lambda) over a [horizon][n] rollout: one thread per battle walks t = horizon - 1 .. 0; loads and stores of one
+// time step are coalesced across the warp.  The arithmetic is the fp32 sequence of the torch loop it replaces
+// (examples/ppo_footsies.py before the value pass moved into the library), operation for operation -- the library is
+// compiled with -fmad=false, so none of it is contracted:
+//   nt = 1 - done[t];  delta = (r[t] + (g * v[t + 1]) * nt) - v[t];  last = delta + (gl * nt) * last;
+//   adv[t] = last;  ret[t] = adv[t] + v[t]
+// The recursion is a dependency chain of `horizon` steps per thread, so the loads of the next kGaeAhead time steps are
+// issued before their arithmetic (the unrolled block below): the chain waits on one memory latency per block, not per step.
+constexpr int kGaeThreads = 256;
+constexpr int kGaeAhead = 8;
+__device__ __forceinline__ void gae_step(float r, uint8_t d, float v, float g, float gl, float &vnext, float &last,
+                                         float *adv, float *ret) {
+    const float nt = d ? 0.0f : 1.0f;                           // = 1 - done for a 0 / 1 flag
+    const float delta = (r + (g * vnext) * nt) - v;
+    last = delta + (gl * nt) * last;
+    *adv = last;
+    *ret = last + v;
+    vnext = v;
+}
+__global__ void __launch_bounds__(kGaeThreads) gae_kernel(const float *__restrict__ rewards, const uint8_t *__restrict__ dones,
+                                                          const float *__restrict__ values, int horizon, int n, float g, float gl,
+                                                          float *__restrict__ adv, float *__restrict__ ret) {
+    const int i = blockIdx.x * kGaeThreads + threadIdx.x;
+    if (i >= n) return;
+    const size_t N = (size_t)n;
+    float vnext = values[(size_t)horizon * N + i], last = 0.0f;
+    int t = horizon - 1;
+    for (; t >= kGaeAhead - 1; t -= kGaeAhead) {
+        float r[kGaeAhead], v[kGaeAhead];
+        uint8_t d[kGaeAhead];
+#pragma unroll
+        for (int u = 0; u < kGaeAhead; u++) {
+            const size_t k = (size_t)(t - u) * N + i;
+            r[u] = rewards[k]; d[u] = dones[k]; v[u] = values[k];
+        }
+#pragma unroll
+        for (int u = 0; u < kGaeAhead; u++) {
+            const size_t k = (size_t)(t - u) * N + i;
+            gae_step(r[u], d[u], v[u], g, gl, vnext, last, adv + k, ret + k);
+        }
+    }
+    for (; t >= 0; t--) {
+        const size_t k = (size_t)t * N + i;
+        gae_step(rewards[k], dones[k], values[k], g, gl, vnext, last, adv + k, ret + k);
+    }
+}
+
 thread_local char g_perr[256] = "";
 
 }  // namespace
@@ -202,6 +279,59 @@ int32_t fg_policy_mlp_sample_p2(const float *obs, const float *scale, const floa
                                 int32_t mirror, int64_t first_env_index, void *stream) {
     return policy_sample_impl(obs, scale, w1, b1, w2, b2, w3, b3, hidden, num_envs, seed, counter, counter_base, actions, logp,
                               nullptr, mirror != 0, first_env_index, stream);
+}
+
+int32_t fg_value_mlp(const float *obs, const float *scale, const float *w1, const float *b1, const float *w2,
+                     const float *b2, const float *w3, const float *b3, int32_t hidden, int64_t rows,
+                     float *values, void *stream) {
+    if (!obs || !scale || !w1 || !b1 || !w2 || !b2 || !w3 || !b3 || !values || rows <= 0) {
+        snprintf(g_perr, sizeof g_perr, "fg_value_mlp: null argument or no rows");
+        return FG_ERR_INVALID_ARGUMENT;
+    }
+    if (hidden != 32 && hidden != 64) {
+        snprintf(g_perr, sizeof g_perr, "fg_value_mlp: hidden size must be 32 or 64");
+        return FG_ERR_INVALID_ARGUMENT;
+    }
+    const PolicyWeights w = { scale, w1, b1, w2, b2, w3, b3 };
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    long long grid = (rows + 32 * kMmaWarps - 1) / (32 * kMmaWarps);
+    if (grid > sms * 4) grid = sms * 4;             // persistent: the weight staging is amortised over many row groups
+    cudaError_t e = cudaSuccess;
+    cudaStream_t s = (cudaStream_t)stream;
+#define FG_VALUE_LAUNCH(HH) do { \
+        constexpr size_t vbytes = PolicyMmaKernelSmem<HH>::kBytes; \
+        static fg::DeviceOnceFlags configured; \
+        e = fg::configure_once_per_device(configured, [] { \
+            return cudaFuncSetAttribute(value_mma_kernel<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)vbytes); }); \
+        if (e == cudaSuccess) value_mma_kernel<HH><<<(unsigned)grid, 32 * kMmaWarps, vbytes, s>>>(obs, w, (long long)rows, values); } while (0)
+    if (hidden == 32) FG_VALUE_LAUNCH(32);
+    else FG_VALUE_LAUNCH(64);
+#undef FG_VALUE_LAUNCH
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        snprintf(g_perr, sizeof g_perr, "fg_value_mlp: %s", cudaGetErrorString(e));
+        return FG_ERR_CUDA;
+    }
+    return FG_OK;
+}
+
+int32_t fg_gae(const float *rewards, const uint8_t *dones, const float *values, int32_t horizon, int32_t num_envs,
+               float gamma, float gamma_lambda, float *advantages, float *returns, void *stream) {
+    if (!rewards || !dones || !values || !advantages || !returns || horizon <= 0 || num_envs <= 0) {
+        snprintf(g_perr, sizeof g_perr, "fg_gae: null argument or empty rollout");
+        return FG_ERR_INVALID_ARGUMENT;
+    }
+    const int grid = (num_envs + kGaeThreads - 1) / kGaeThreads;
+    gae_kernel<<<grid, kGaeThreads, 0, (cudaStream_t)stream>>>(rewards, dones, values, horizon, num_envs, gamma, gamma_lambda,
+                                                               advantages, returns);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        snprintf(g_perr, sizeof g_perr, "fg_gae: %s", cudaGetErrorString(e));
+        return FG_ERR_CUDA;
+    }
+    return FG_OK;
 }
 
 }  // extern "C"

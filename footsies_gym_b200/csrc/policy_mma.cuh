@@ -130,8 +130,12 @@ constexpr float kTwoLog2e = 2.8853900432586669921875f;
 
 // Stage one weight set (torch.nn.Linear layout: W[out][in]) as pre-split B fragments.  Called by every thread of the CTA
 // (nthreads a multiple of 32); the FP16 path contains two CTA barriers (the per-matrix maximum that fixes the scale).
-template <int H>
+// NOUT = real output rows of layer 3 (W3 [NOUT][H], b3 [NOUT]): 8 for the policy's logits, 1 for a value head.  The
+// remaining rows of the 8-wide output tile are staged as zeros and never read from the caller's pointers, and the W3 scale
+// comes from the real rows alone; for NOUT = 8 every added condition is constant and the code is the policy's as before.
+template <int H, int NOUT = 8>
 __device__ __forceinline__ void policy_mma_stage(float *sm, const PolicyWeights &p, int tid, int nthreads) {
+    static_assert(NOUT >= 1 && NOUT <= 8, "layer 3 has one n-tile of 8 outputs");
     using L = PolicyMmaSmem<H>;
     constexpr int NT = L::NT;
     float4 *frag = reinterpret_cast<float4 *>(sm);
@@ -152,7 +156,7 @@ __device__ __forceinline__ void policy_mma_stage(float *sm, const PolicyWeights 
     {
         uint32_t m2 = 0u, m3 = 0u;                                  // |w| as bits: ordered like the values
         for (int i = tid; i < H * H; i += nthreads) m2 = max(m2, __float_as_uint(p.w2[i]) & 0x7fffffffu);
-        for (int i = tid; i < 8 * H; i += nthreads) m3 = max(m3, __float_as_uint(p.w3[i]) & 0x7fffffffu);
+        for (int i = tid; i < NOUT * H; i += nthreads) m3 = max(m3, __float_as_uint(p.w3[i]) & 0x7fffffffu);
         m2 = __reduce_max_sync(0xffffffffu, m2); m3 = __reduce_max_sync(0xffffffffu, m3);
         if ((tid & 31) == 0) { atomicMax(&smax[0], m2); atomicMax(&smax[1], m3); }
     }
@@ -179,11 +183,15 @@ __device__ __forceinline__ void policy_mma_stage(float *sm, const PolicyWeights 
     // layer 3: one n-tile (the 8 logits), n = g
     for (int i = tid; i < L::KT * 32; i += nthreads) {
         const int kt = i >> 5, lane = i & 31, g = lane >> 2, t = lane & 3;
-        put16(L::kW3 + i, p.w3 + g * H + 16 * kt + 2 * t, s3);
+        if (NOUT < 8 && g >= NOUT) hfrag[L::kW3 + i] = make_uint4(0u, 0u, 0u, 0u);
+        else put16(L::kW3 + i, p.w3 + g * H + 16 * kt + 2 * t, s3);
     }
     // biases of the scaled layers in accumulator units
     for (int i = tid; i < H; i += nthreads) { sm[L::kB1 + i] = p.b1[i]; sm[L::kB2 + i] = p.b2[i] * (kActScale * s2); }
-    if (tid < 8) { sm[L::kB3 + tid] = p.b3[tid] * (kActScale * s3); sm[L::kScale + tid] = p.scale[tid]; }
+    if (tid < 8) {
+        sm[L::kB3 + tid] = (NOUT == 8 || tid < NOUT) ? p.b3[tid] * (kActScale * s3) : 0.0f;
+        sm[L::kScale + tid] = p.scale[tid];
+    }
     if (tid == 0) {
         sm[L::kInv2] = __uint_as_float((uint32_t)(e2 - 20) << 23);
         sm[L::kInv3] = __uint_as_float((uint32_t)(e3 - 20) << 23);
@@ -202,14 +210,16 @@ __device__ __forceinline__ void policy_mma_stage(float *sm, const PolicyWeights 
     // layer 3: one n-tile (the 8 logits), n = g
     for (int i = tid; i < NT * 32; i += nthreads) {
         const int kt = i >> 5, lane = i & 31, g = lane >> 2, t = lane & 3;
-        put(L::kW3 + i, p.w3[g * H + 8 * kt + 2 * t], p.w3[g * H + 8 * kt + 2 * t + 1]);
+        if (NOUT < 8 && g >= NOUT) frag[L::kW3 + i] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        else put(L::kW3 + i, p.w3[g * H + 8 * kt + 2 * t], p.w3[g * H + 8 * kt + 2 * t + 1]);
     }
     for (int i = tid; i < H; i += nthreads) { sm[L::kB1 + i] = p.b1[i]; sm[L::kB2 + i] = p.b2[i]; }
-    if (tid < 8) { sm[L::kB3 + tid] = p.b3[tid]; sm[L::kScale + tid] = p.scale[tid]; }
+    if (tid < 8) { sm[L::kB3 + tid] = (NOUT == 8 || tid < NOUT) ? p.b3[tid] : 0.0f; sm[L::kScale + tid] = p.scale[tid]; }
 #endif
 }
 
-// The 8 logits of the warp's 16 MT battles.  obs_rows: the battles' raw observation rows ([16 MT][8] floats, shared or
+// The 8 logits of the warp's 16 MT battles (for a weight set staged with NOUT < 8: its NOUT outputs in columns 0 .. NOUT - 1,
+// zeros after them).  obs_rows: the battles' raw observation rows ([16 MT][8] floats, shared or
 // global memory); lg_rows: [16 MT][8] floats of shared memory private to the warp, where row r receives battle r's logits
 // (the caller reads its own row after the __syncwarp at the end).  MIRROR shows the network the observation as the other
 // player sees it (policy_mirror_obs: per-player fields swap, positions change sign).

@@ -15,6 +15,10 @@ Three policy paths:
     registers from the first step to the last and alternates policy inference and the frame update; bit-identical
     to the per-step path.
 
+With a value network (`value=`), collect() also returns what a PPO update consumes besides the rollout itself: the values
+of all horizon + 1 observation rows (one fg_value_mlp launch for an `MLPValue` with hidden 32 / 64, else one call of the
+torch callable) and GAE advantages / returns (one fg_gae launch), after the rollout on the same stream.
+
 PyTorch is plumbing here (parameters, buffers, CUDA graph); the simulator step inside the loop is fg_step.
 """
 import ctypes as C
@@ -86,6 +90,90 @@ class MLPPolicy(torch.nn.Module):
             raise _capi.FootsiesLibraryError(lib.fg_policy_last_error().decode())
 
 
+class MLPValue(torch.nn.Module):
+    """Value network 8 -> hidden -> hidden -> 1 (tanh) on the observation times the same `scale` as MLPPolicy.
+    hidden in {32, 64} can be run by the fused kernel (fused_values); any hidden size runs as a torch module."""
+
+    def __init__(self, hidden: int = 64):
+        super().__init__()
+        self.hidden = int(hidden)
+        self.register_buffer("scale", torch.tensor(_OBS_SCALE, dtype=torch.float32))
+        self.net = torch.nn.Sequential(torch.nn.Linear(8, hidden), torch.nn.Tanh(), torch.nn.Linear(hidden, hidden),
+                                       torch.nn.Tanh(), torch.nn.Linear(hidden, 1))
+
+    def forward(self, obs: torch.Tensor) -> torch.Tensor:
+        """obs [N, 8] -> values [N]"""
+        return self.net(obs * self.scale).squeeze(-1)
+
+    def fused_values(self, obs_rows: torch.Tensor, out: torch.Tensor):
+        """One launch of fg_value_mlp on the current stream: out (float32, one value per observation row) receives the
+        values of obs_rows (float32 [..., 8], e.g. a whole [horizon + 1, N, 8] rollout buffer).  Agrees with forward() to
+        ~1e-5 relative (tensor-core path with split operands, not torch's fp32 GEMM)."""
+        if self.hidden not in (32, 64):
+            raise ValueError(f"fused_values needs hidden 32 or 64 (got {self.hidden}): use the module itself")
+        lib = _capi.load()
+        l1, l2, l3 = self.net[0], self.net[2], self.net[4]
+        ts = [obs_rows, self.scale, l1.weight, l1.bias, l2.weight, l2.bias, l3.weight, l3.bias]
+        for t in ts:
+            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != obs_rows.device:
+                raise ValueError("fused value inference needs contiguous float32 tensors on one device")
+        if obs_rows.device.type != "cuda":
+            raise ValueError("fused value inference needs CUDA tensors")
+        if obs_rows.dim() < 1 or obs_rows.shape[-1] != 8:
+            raise ValueError("obs_rows must have 8 features in its last dimension")
+        rows = obs_rows.numel() // 8
+        if out.dtype != torch.float32 or not out.is_contiguous() or out.device != obs_rows.device or out.numel() != rows:
+            raise ValueError(f"out must be a contiguous float32 tensor of {rows} values on the observations' device")
+        rc = lib.fg_value_mlp(*[C.c_void_p(t.data_ptr()) for t in ts], self.hidden, rows, C.c_void_p(out.data_ptr()),
+                              C.c_void_p(torch.cuda.current_stream(obs_rows.device).cuda_stream))
+        if rc != 0:
+            raise _capi.FootsiesLibraryError(lib.fg_policy_last_error().decode())
+
+
+def compute_gae(rewards: torch.Tensor, dones: torch.Tensor, values: torch.Tensor, gamma: float, gae_lambda: float,
+                advantages: Optional[torch.Tensor] = None, returns: Optional[torch.Tensor] = None):
+    """GAE advantages and returns of a [horizon, N] rollout in one launch of fg_gae on the current stream.
+
+    rewards float32 [h, N]; dones bool / uint8 [h, N] (a done at step t cuts the bootstrap from t + 1); values float32
+    [h + 1, N] (values[h]: the observation after the last step); all contiguous on one CUDA device.  advantages / returns:
+    optional float32 [h, N] outputs (allocated when None).  Returns (advantages, returns).  Bit-identical to the torch loop
+        last = 0
+        for t in reversed(range(h)):
+            nonterm = 1.0 - dones[t].float()
+            delta = rewards[t] + gamma * values[t + 1] * nonterm - values[t]
+            last = delta + gamma * gae_lambda * nonterm * last
+            advantages[t] = last
+        returns = advantages + values[:h]"""
+    if rewards.dim() != 2:
+        raise ValueError("rewards must be [horizon, N]")
+    h, n = rewards.shape
+    if h == 0 or n == 0:
+        raise ValueError("empty rollout")
+    if rewards.device.type != "cuda":
+        raise ValueError("compute_gae needs CUDA tensors")
+    dev = rewards.device
+    if advantages is None:
+        advantages = torch.empty((h, n), dtype=torch.float32, device=dev)
+    if returns is None:
+        returns = torch.empty((h, n), dtype=torch.float32, device=dev)
+    for name, t, dtypes, shape in (("rewards", rewards, (torch.float32,), (h, n)),
+                                   ("dones", dones, (torch.bool, torch.uint8), (h, n)),
+                                   ("values", values, (torch.float32,), (h + 1, n)),
+                                   ("advantages", advantages, (torch.float32,), (h, n)),
+                                   ("returns", returns, (torch.float32,), (h, n))):
+        if t.dtype not in dtypes or tuple(t.shape) != shape or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"{name} must be a contiguous {' / '.join(str(d) for d in dtypes)} tensor of shape {shape} "
+                             f"on {dev} (got {t.dtype} {tuple(t.shape)} on {t.device})")
+    lib = _capi.load()
+    ptr = lambda t: C.c_void_p(t.data_ptr())   # noqa: E731
+    # gamma * gae_lambda in double, then rounded once to fp32: what torch does with the Python scalar of the loop above
+    rc = lib.fg_gae(ptr(rewards), ptr(dones), ptr(values), h, n, float(gamma), float(gamma) * float(gae_lambda),
+                    ptr(advantages), ptr(returns), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+    if rc != 0:
+        raise _capi.FootsiesLibraryError(lib.fg_policy_last_error().decode())
+    return advantages, returns
+
+
 def mirror_obs(obs: torch.Tensor) -> torch.Tensor:
     """The observation [N, 8] as P2 sees it: per-player fields swapped, positions negated."""
     m = obs[:, [1, 0, 3, 2, 5, 4, 7, 6]].clone()
@@ -101,17 +189,22 @@ class RolloutCollector:
     """Collects `horizon` steps of (obs, action, log-prob, reward, done) for every env of one GPU, entirely on device.
 
     Buffers (overwritten by every collect()): obs [horizon + 1, N, 8] (obs[t] is what the policy saw at step t, obs[-1]
-    the observation after the last step), actions uint8 [horizon, N], logp / rewards float32 [horizon, N], dones bool."""
+    the observation after the last step), actions uint8 [horizon, N], logp / rewards float32 [horizon, N], dones bool;
+    with a value network also values float32 [horizon + 1, N] (of every obs row) and advantages / returns float32
+    [horizon, N] (GAE with gamma, gae_lambda; see compute_gae)."""
 
     def __init__(self, env: FootsiesEnv, policy: Callable[[torch.Tensor], torch.Tensor], horizon: int = 128,
                  use_cuda_graph: bool = True, fused=None, seed: int = 0,
-                 opponent_policy: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, mirror_opponent: bool = False):
+                 opponent_policy: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, mirror_opponent: bool = False,
+                 value: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, gamma: float = 0.99, gae_lambda: float = 0.95):
         """fused: None / True = the most fused path available ("horizon", else "step", else torch ops for a policy that
         is not an MLPPolicy); False = torch ops; "step" / "horizon" = that path or an error.
         opponent_policy: a second policy for P2 (self-play rollouts; the env must take P2's actions from step(), i.e.
         opponent="self_play" / "remote").  It sees the same observation as the reference's `opponent(obs, info)`
         callable (footsies.py:522-527), or its mirror image with mirror_opponent=True (then `policy` itself can be passed
-        again: one network plays both sides).  Its actions / log-probabilities are collected in actions_p2 / logp_p2."""
+        again: one network plays both sides).  Its actions / log-probabilities are collected in actions_p2 / logp_p2.
+        value: a value network, `value(obs[M, 8]) -> [M]` or `[M, 1]`; an MLPValue with hidden 32 / 64 runs on the fused
+        kernel (fg_value_mlp).  The policy path is chosen as without it.  Values and advantages are P1's."""
         if env.by_example:
             raise ValueError("the policy drives P1: create the env with by_example=False")
         if env.frame_delay:
@@ -149,6 +242,13 @@ class RolloutCollector:
             self.actions_p2 = torch.zeros((h, n), dtype=torch.uint8, device=dev)
             self.logp_p2 = torch.zeros((h, n), dtype=torch.float32, device=dev)
             self._mirror_action = torch.tensor(_MIRROR_ACTION, dtype=torch.uint8, device=dev)
+        self.value, self.gamma, self.gae_lambda = value, float(gamma), float(gae_lambda)
+        self.values = self.advantages = self.returns = None
+        if value is not None:
+            self._fused_value = isinstance(value, MLPValue) and value.hidden in (32, 64)
+            self.values = torch.zeros((h + 1, n), dtype=torch.float32, device=dev)
+            self.advantages = torch.zeros((h, n), dtype=torch.float32, device=dev)
+            self.returns = torch.zeros((h, n), dtype=torch.float32, device=dev)
         self._seed = int(seed)
         self._drawn = torch.zeros(1, dtype=torch.int64, device=dev)   # policy steps taken so far (device side: graph replays bump it)
         self._graph = None
@@ -180,8 +280,24 @@ class RolloutCollector:
         _capi.check(env._lib.fg_rollout_mlp(env._handle, C.byref(r), env._stream()))
         self._drawn.add_(self.horizon)
 
+    def _values_and_gae(self):
+        """Values of all (horizon + 1) x N observation rows, then GAE: two launches on the current stream."""
+        if self._fused_value:
+            self.value.fused_values(self.obs, self.values)
+        else:
+            v = self.value(self.obs.view(-1, 8))
+            if v.dim() == 2 and v.shape[1] == 1:
+                v = v.squeeze(1)
+            self.values.view(-1).copy_(v)
+        compute_gae(self.rewards, self.dones, self.values, self.gamma, self.gae_lambda, self.advantages, self.returns)
+
     @torch.no_grad()
     def _one_horizon(self):
+        self._rollout()
+        if self.value is not None:
+            self._values_and_gae()
+
+    def _rollout(self):
         env, h = self.env, self.horizon
         if self.mode == "horizon":
             return self._horizon_launch()
@@ -215,7 +331,8 @@ class RolloutCollector:
         self._drawn.add_(h)
 
     def collect(self):
-        """Runs one horizon; returns the rollout buffers (views, overwritten by the next call)."""
+        """Runs one horizon (and with a value network its values and GAE); returns the rollout buffers (views,
+        overwritten by the next call)."""
         dev = self.env.device
         if not self.use_cuda_graph or self.mode == "horizon":      # one launch: nothing for a graph to save
             self._one_horizon()
@@ -235,4 +352,6 @@ class RolloutCollector:
                "dones": self.dones, "last_obs": self.obs[self.horizon]}
         if self.opponent_policy is not None:
             out.update(actions_p2=self.actions_p2, logp_p2=self.logp_p2)
+        if self.value is not None:
+            out.update(values=self.values, advantages=self.advantages, returns=self.returns)
         return out

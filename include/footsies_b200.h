@@ -23,7 +23,8 @@ extern "C" {
 #endif
 
 /* 2 (round 2): fg_env_state.p1_bot_memory, first_env_index argument of fg_policy_mlp_sample[_p2], packed host layout
- * (fg_packed_result, fg_step_host_packed, fg_reset_host_packed, fg_packed_reward_table), fg_host_alloc / fg_host_free */
+ * (fg_packed_result, fg_step_host_packed, fg_reset_host_packed, fg_packed_reward_table), fg_host_alloc / fg_host_free.
+ * Added since, backward compatible (new entry points only, so still 2): fg_value_mlp, fg_gae. */
 #define FG_ABI_VERSION 2
 
 typedef enum {
@@ -276,6 +277,30 @@ typedef struct {
     int32_t reserved1;
 } fg_rollout_buffers;
 int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream);
+
+/* Critic side of an actor-critic (PPO) rollout, for any source of rollout buffers.  Handle-free like fg_policy_mlp_sample;
+ * errors are reported through fg_policy_last_error().  All pointers are DEVICE pointers.
+ *
+ * fg_value_mlp: values[i] = V(obs[i] * scale) for a value network obs * scale -> Linear(8, H) -> tanh -> Linear(H, H) ->
+ * tanh -> Linear(H, 1), for rows i = 0 .. rows - 1 of obs [rows][8] (e.g. a whole [horizon + 1][num_envs][8] rollout
+ * buffer: rows may exceed INT32_MAX).  Weights row-major [out][in] like torch.nn.Linear: w1 [H][8], b1 [H], w2 [H][H],
+ * b2 [H], w3 [1][H], b3 [1]; scale [8].  hidden must be 32 or 64.  It stands in for the separate torch value MLP of the
+ * PPO example (examples/ppo_footsies.py before this entry point), on the tensor-core path of the policy kernel: agrees
+ * with torch's fp32 forward to ~1e-5 relative. */
+int32_t fg_value_mlp(const float *obs, const float *scale, const float *w1, const float *b1, const float *w2,
+                     const float *b2, const float *w3, const float *b3, int32_t hidden, int64_t rows,
+                     float *values, void *stream);
+/* fg_gae: generalised advantage estimation over rewards [horizon][num_envs], dones [horizon][num_envs] (0 / 1 flags, e.g.
+ * fg_rollout_buffers.dones) and values [horizon + 1][num_envs] (values[horizon] = the value of the observation after the
+ * last step); writes advantages and returns [horizon][num_envs].  A done at step t cuts the bootstrap from t + 1 (the
+ * autoreset step after it is an ordinary transition).  Per battle, for t = horizon - 1 .. 0, in fp32 and in this order:
+ *   nt = 1 - dones[t];  delta = (rewards[t] + (gamma * values[t + 1]) * nt) - values[t];
+ *   last = delta + (gamma_lambda * nt) * last  (last = 0 before t = horizon - 1);  advantages[t] = last;
+ *   returns[t] = advantages[t] + values[t]
+ * -- the torch loop of the PPO example (examples/ppo_footsies.py before this entry point) operation for operation, so the
+ * results are bit-identical to it when gamma_lambda is gamma * lambda rounded to float from the double product. */
+int32_t fg_gae(const float *rewards, const uint8_t *dones, const float *values, int32_t horizon, int32_t num_envs,
+               float gamma, float gamma_lambda, float *advantages, float *returns, void *stream);
 
 #ifdef __cplusplus
 }
