@@ -2,6 +2,7 @@
 """PPO against the in-game bot, entirely on the GPU (BASELINE.json configs[4] in use).
 
     python examples/ppo_footsies.py [--envs 16384] [--horizon 128] [--iters 40] [--frame-skip 1] [--self-play]
+                                    [--pool K --snapshot-every S]
     torchrun --nproc-per-node 8 examples/ppo_footsies.py          # one process per GPU, gradients all-reduced
 
 Rollouts come from footsies_gym_b200.rollout.RolloutCollector: the fused policy kernel samples actions from the
@@ -13,6 +14,11 @@ network's parameters are updated in place, so the next rollout reads the new wei
 Prints the win rate against the bot per iteration (from the kernel's own episode statistics).
 With --self-play the training rollouts are played against the same network on the mirrored observation (still one
 launch per horizon) and the win rate against the in-game bot comes from a separate evaluation rollout per iteration.
+With --self-play --pool K the opponent is a pool of K networks sharing the battles equally (fg_rollout_mlp_pool, still
+one launch per horizon): member 0 is the live policy, the other K - 1 slots hold frozen snapshots of it, refreshed one
+slot at a time in round-robin order every S iterations (all start as the initial policy).  Each iteration also prints the
+win rate against every member, from the kernel's per-member counters (all-reduced over the ranks, which use the same
+shares).
 """
 import argparse
 import os
@@ -42,7 +48,14 @@ def main():
     ap.add_argument("--clip", type=float, default=0.2)
     ap.add_argument("--entropy", type=float, default=0.01)
     ap.add_argument("--self-play", action="store_true", help="train against the same network playing the mirrored side")
+    ap.add_argument("--pool", type=int, default=0, help="with --self-play: play against a pool of this many networks "
+                    "(the live policy + K - 1 snapshots)")
+    ap.add_argument("--snapshot-every", type=int, default=5, help="iterations between two snapshots into the pool")
     a = ap.parse_args()
+    if a.pool and not a.self_play:
+        ap.error("--pool needs --self-play")
+    if a.pool < 0 or a.pool > 16 or a.snapshot_every < 1:
+        ap.error("--pool must be in 1 .. 16 and --snapshot-every positive")
 
     rank, local_rank, world = env_rank_world()
     dev = torch.device("cuda", local_rank)
@@ -59,9 +72,16 @@ def main():
         for p in params:
             dist.broadcast(p.data, 0)
     opt = torch.optim.Adam(params, lr=a.lr)
+    pool = None
+    if a.pool:
+        pool = [policy] + [MLPPolicy(64).to(dev) for _ in range(a.pool - 1)]
+        for m in pool[1:]:
+            m.load_state_dict(policy.state_dict())
+            m.requires_grad_(False)
     col = RolloutCollector(env, policy, horizon=a.horizon, use_cuda_graph=True, seed=rank,
-                           opponent_policy=policy if a.self_play else None, mirror_opponent=a.self_play,
-                           value=value, gamma=a.gamma, gae_lambda=a.lam)
+                           opponent_policy=policy if a.self_play and not a.pool else None, mirror_opponent=a.self_play,
+                           opponent_pool=pool, value=value, gamma=a.gamma, gae_lambda=a.lam)
+    next_slot = 1
     eval_env = eval_col = None
     if a.self_play:                       # the yardstick stays the in-game bot
         eval_env = make_sharded_env(a.envs * world, frame_skip=a.frame_skip, seed=1)
@@ -69,6 +89,7 @@ def main():
     n, h = env.num_envs, a.horizon
     stat_env = eval_env if a.self_play else env
     prev = stat_env.episode_stats()
+    prev_pool = col.opponent_pool_stats() if pool else None
     t_roll = t_upd = 0.0
     for it in range(a.iters):
         t0 = time.perf_counter()
@@ -119,9 +140,21 @@ def main():
         ep = st["episodes"] - prev["episodes"]
         wins = st["p1_wins"] - prev["p1_wins"]
         prev = st
+        pool_msg = ""
+        if pool:
+            cur = col.opponent_pool_stats()
+            d = cur - prev_pool                              # [K, 4] this iteration: episodes, P1 wins, P2 wins, double KOs
+            prev_pool = cur
+            if world > 1:
+                dist.all_reduce(d)
+            d = d.cpu()
+            pool_msg = "  win rate vs pool [" + " ".join(f"{int(w) / max(int(e), 1):.2f}" for e, w in d[:, :2].tolist()) + "]"
+            if (it + 1) % a.snapshot_every == 0 and a.pool > 1:
+                pool[next_slot].load_state_dict(policy.state_dict())     # played from the next collect() on
+                next_slot = next_slot % (a.pool - 1) + 1
         if rank == 0:
             print(f"iter {it:3d}  episodes {ep:8d}  win rate vs bot {wins / max(ep, 1):.3f}  mean reward/step {float(rew.mean()):+.4f}  "
-                  f"rollout {frames / (t1 - t0) / 1e6:8.1f} M env-frames/s  update {t2 - t1:.2f} s", flush=True)
+                  f"rollout {frames / (t1 - t0) / 1e6:8.1f} M env-frames/s  update {t2 - t1:.2f} s{pool_msg}", flush=True)
     if rank == 0:
         print(f"total: rollouts {t_roll:.1f} s, updates {t_upd:.1f} s")
     if world > 1:

@@ -46,6 +46,20 @@ class FgRolloutBuffers(C.Structure):
                 ("actions_p2", C.c_void_p), ("logp_p2", C.c_void_p), ("p2_mirror", C.c_int32), ("reserved1", C.c_int32)]
 
 
+FG_POOL_MAX = 16
+FG_POOL_BLOCK = 128
+
+
+class FgMlpWeights(C.Structure):
+    _fields_ = [("scale", C.c_void_p), ("w1", C.c_void_p), ("b1", C.c_void_p), ("w2", C.c_void_p), ("b2", C.c_void_p),
+                ("w3", C.c_void_p), ("b3", C.c_void_p)]
+
+
+class FgOpponentPool(C.Structure):
+    _fields_ = [("struct_size", C.c_int32), ("count", C.c_int32), ("member", FgMlpWeights * FG_POOL_MAX),
+                ("end", C.c_int64 * FG_POOL_MAX), ("stats", C.c_void_p)]
+
+
 class FgFighterState(C.Structure):
     _fields_ = [("pos_x", C.c_float), ("velocity_x", C.c_float), ("action_id", C.c_int32),
                 ("action_frame", C.c_int32), ("hitstun", C.c_int32), ("guard", C.c_int32), ("vital", C.c_int32),
@@ -118,7 +132,7 @@ EXPORTS = ["fg_abi_version", "fg_last_error", "fg_algorithmic_bytes_per_env_step
            "fg_reset_host_compact", "fg_packed_reward_table", "fg_step_host_packed", "fg_reset_host_packed", "fg_host_alloc",
            "fg_host_free", "fg_delay_ring_step", "fg_get_state",
            "fg_set_state", "fg_read_stats", "fg_launch_count", "fg_policy_mlp_sample", "fg_policy_mlp_sample_p2", "fg_policy_last_error",
-           "fg_rollout_mlp", "fg_value_mlp", "fg_gae"]
+           "fg_rollout_mlp", "fg_rollout_mlp_pool", "fg_value_mlp", "fg_gae"]
 
 
 def load(build_if_missing=True):
@@ -187,6 +201,8 @@ def load(build_if_missing=True):
     L.fg_policy_last_error.restype = C.c_char_p
     L.fg_rollout_mlp.restype = i32
     L.fg_rollout_mlp.argtypes = [vp, C.POINTER(FgRolloutBuffers), vp]
+    L.fg_rollout_mlp_pool.restype = i32
+    L.fg_rollout_mlp_pool.argtypes = [vp, C.POINTER(FgRolloutBuffers), C.POINTER(FgOpponentPool), vp]
     L.fg_value_mlp.restype = i32
     L.fg_value_mlp.argtypes = [vp] * 8 + [i32, i64, vp, vp]
     L.fg_gae.restype = i32

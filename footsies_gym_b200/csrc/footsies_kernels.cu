@@ -773,6 +773,61 @@ int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) 
     return FG_OK;
 }
 
+int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, void *stream) {
+    if (!pool || pool->struct_size != (int32_t)sizeof(fg_opponent_pool))
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool is null or its struct_size does not match%s");
+    if (int rc = check_bound(h)) return rc;
+    if (!r || r->struct_size != (int32_t)sizeof(fg_rollout_buffers))
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers is null or its struct_size does not match%s");
+    if (h->cfg.p1_bot || !h->cfg.autoreset || h->buf.step_mask)
+        return fail(FG_ERR_INVALID_STATE, "fg_rollout_mlp_pool needs P1 = policy, autoreset on, no step mask%s");
+    if (h->cfg.p2_bot)
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_pool needs p2_bot = 0: the pool plays P2 (the in-game bot cannot be a member)%s");
+    if (pool->count < 1 || pool->count > FG_POOL_MAX) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.count must be in 1..16%s");
+    const int64_t n = h->cfg.num_envs;
+    for (int m = 0; m < pool->count; m++) {
+        const int64_t lo = m ? pool->end[m - 1] : 0, e = pool->end[m];
+        if (e < lo || e > n) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end must be non-decreasing and at most num_envs%s");
+        if (e % FG_POOL_BLOCK && e != n)
+            return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end: every boundary must be a multiple of FG_POOL_BLOCK (128) or num_envs%s");
+        const fg_mlp_weights &w = pool->member[m];
+        if (!w.scale || !w.w1 || !w.b1 || !w.w2 || !w.b2 || !w.w3 || !w.b3)
+            return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool: null member weight pointer%s");
+        if ((uintptr_t)w.w2 & 15u) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool: member w2 must be 16-byte aligned%s");
+    }
+    if (pool->end[pool->count - 1] != n) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end[count - 1] must be num_envs%s");
+    if ((uintptr_t)pool->stats & 7u) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.stats must be 8-byte aligned%s");
+    if (r->hidden != 32 && r->hidden != 64 && r->hidden != 128)
+        return fail(FG_ERR_INVALID_ARGUMENT, "hidden size must be 32, 64 or 128 (the learner's and every member's)%s");
+    if (r->horizon < 1) return fail(FG_ERR_INVALID_ARGUMENT, "horizon must be positive%s");
+    if (!r->scale || !r->w1 || !r->b1 || !r->w2 || !r->b2 || !r->w3 || !r->b3 || !r->obs || !r->actions || !r->logp || !r->rewards ||
+        !r->dones || !r->actions_p2 || !r->logp_p2)
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers: null pointer (actions_p2 and logp_p2 are required)%s");
+    if (((uintptr_t)r->obs & 15u) || ((uintptr_t)r->w2 & 15u)) return fail(FG_ERR_INVALID_ARGUMENT, "obs and w2 must be 16-byte aligned%s");
+    CUDA_TRY(cudaSetDevice(h->cfg.device));
+    RolloutPoolParams rp;
+    rp.sim = make_params(h);
+    rp.w = { r->scale, r->w1, r->b1, r->w2, r->b2, r->w3, r->b3 };
+    rp.seed = r->seed; rp.counter_base = (const unsigned long long *)r->counter_base;
+    rp.hidden = r->hidden; rp.horizon = r->horizon;
+    rp.obs = (float4 *)r->obs; rp.actions = r->actions; rp.logp = r->logp; rp.rewards = r->rewards; rp.dones = r->dones;
+    rp.p2_policy = 1; rp.p2_mirror = r->p2_mirror != 0;
+    rp.w_p2 = {};
+    rp.seed_p2 = r->p2_seed; rp.actions_p2 = r->actions_p2; rp.logp_p2 = r->logp_p2;
+    for (int m = 0; m < FG_POOL_MAX; m++) {
+        const bool used = m < pool->count;
+        const fg_mlp_weights &w = pool->member[used ? m : 0];
+        rp.pool.member[m] = { w.scale, w.w1, w.b1, w.w2, w.b2, w.w3, w.b3 };
+        rp.pool.end[m] = used ? pool->end[m] : n;
+    }
+    rp.pool.count = pool->count;
+    rp.pool.stats = (unsigned long long *)pool->stats;
+    CUDA_TRY(launch_rollout_pool(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
+    h->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return FG_OK;
+}
+
 int64_t fg_launch_count(fg_handle *h) { return h ? h->launches : 0; }
 
 }  // extern "C"

@@ -16,8 +16,14 @@
 // co-resident CTA half a step late so that simulator and policy phases interleave: no measurable effect for any delay;
 // one CTA per SM runs a step in 4.7 us, two in 6.5 us, so co-residency already overlaps most of the work.  Removed.)
 // Results are bit-identical to the per-step path (tests/test_rollout.py).
+// Opponent pool (fg_rollout_mlp_pool, POOL = true): P2 is played by up to FG_POOL_MAX networks, member m on the battles
+// [end[m - 1], end[m]).  The boundaries are multiples of FG_POOL_BLOCK, a multiple of every CTA's battle count, so a CTA
+// stages one member's weights in the single P2 policy's place and runs the same horizon loop; its final statistics flush
+// also lands in that member's counters.  Every range equals a single-opponent rollout of just those battles
+// (tests/test_opponent_pool.py); the POOL = false instantiations are the kernels as they were.
 // Compiled with -fmad=false like the step kernel; the policy arithmetic uses explicit fmaf.
 #include <stdlib.h>
+#include <type_traits>
 
 #include "rollout_kernel.h"
 #include "policy_mma.cuh"
@@ -38,13 +44,40 @@ struct RolloutSmem {
     static constexpr size_t kBytes = kStats + sizeof(unsigned long long) * FG_STAT_COUNT;
 };
 
-template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP>
-__global__ void __launch_bounds__(32 * W) rollout_kernel(const RolloutParams rp) {
+// ---- opponent pool (fg_rollout_mlp_pool): a CTA's P2 weights are those of the member whose range holds its battles ----
+template <bool POOL> struct RolloutArgs { using type = RolloutParams; };
+template <> struct RolloutArgs<true> { using type = RolloutPoolParams; };
+
+// member of the CTA whose first battle is `first`: the number of boundaries end[0 .. count - 2] at or below it (end is
+// non-decreasing and first < n = end[count - 1]).  Unrolled with constant indices so that the parameter arrays are read
+// from the constant bank instead of being copied to local memory for a dynamic index.
+__device__ __forceinline__ int pool_member(const RolloutPool &pool, long long first) {
+    int m = 0;
+#pragma unroll
+    for (int k = 0; k < FG_POOL_MAX - 1; k++) m += (k < pool.count - 1 && first >= pool.end[k]) ? 1 : 0;
+    return m;
+}
+__device__ __forceinline__ PolicyWeights pool_weights(const RolloutPool &pool, int m) {
+    PolicyWeights w = pool.member[0];
+#pragma unroll
+    for (int k = 1; k < FG_POOL_MAX; k++)
+        if (k == m) w = pool.member[k];
+    return w;
+}
+// after the CTA's final statistics flush (and its barrier): the member's episodes, P1 wins, P2 wins, double KOs
+__device__ __forceinline__ void pool_flush(const RolloutPool &pool, int m, const unsigned long long *s_stats, int tid) {
+    static_assert(FG_STAT_EPISODES == 0 && FG_STAT_P1_WINS == 1 && FG_STAT_P2_WINS == 2 && FG_STAT_DOUBLE_KO == 3, "stats[m][4] order");
+    if (pool.stats && tid < 4 && s_stats[tid]) atomicAdd(&pool.stats[(size_t)m * 4 + tid], s_stats[tid]);
+}
+
+template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL = false>
+__global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutArgs<POOL>::type rp) {
     using SM = RolloutSmem<H, E, W, P2POL>;
     using PL = typename SM::PL;
     constexpr bool kP2Bot = !P2POL;                             // P2 = in-game bot (needs the RNG plane) or the second policy
     constexpr int kEnvs = SM::kEnvs, kRollThreads = 32 * W;
     static_assert(kEnvs <= kRollThreads, "one simulator thread per battle");
+    static_assert(!POOL || (P2POL && FG_POOL_BLOCK % kEnvs == 0), "a pool CTA plays against one member");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Tables &Tw = *reinterpret_cast<Tables *>(smem_raw + SM::kTables);
     const Tables &T = Tw;
@@ -64,7 +97,11 @@ __global__ void __launch_bounds__(32 * W) rollout_kernel(const RolloutParams rp)
 
     load_tables(&Tw, p.tables);
     policy_stage_bcast<H, kEnvs, W>(pw, rp.w, tid, kRollThreads);
-    if (P2POL) policy_stage_bcast<H, kEnvs, W>(pw2, rp.w_p2, tid, kRollThreads);
+    int member = 0;
+    if constexpr (POOL) {
+        member = pool_member(rp.pool, base);
+        policy_stage_bcast<H, kEnvs, W>(pw2, pool_weights(rp.pool, member), tid, kRollThreads);
+    } else if (P2POL) policy_stage_bcast<H, kEnvs, W>(pw2, rp.w_p2, tid, kRollThreads);
     if (tid < FG_STAT_COUNT) s_stats[tid] = 0ull;
     Env e;
     if (valid) load_env<kP2Bot>(p, i, e);
@@ -185,6 +222,7 @@ __global__ void __launch_bounds__(32 * W) rollout_kernel(const RolloutParams rp)
     }
     __syncthreads();
     if (tid < FG_STAT_COUNT && s_stats[tid]) atomicAdd(&p.stats[tid], s_stats[tid]);
+    if constexpr (POOL) pool_flush(rp.pool, member, s_stats, tid);
 }
 
 // ---- tensor-core version (H <= 64): every WARP owns 16 MT battles for the whole horizon -- policy (policy_mma.cuh: mma.sync
@@ -210,11 +248,13 @@ struct RolloutMmaSmem {
 #ifndef FG_ROLLOUT_MT2_MIN_BLOCKS
 #define FG_ROLLOUT_MT2_MIN_BLOCKS 1
 #endif
-template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP>
-__global__ void __launch_bounds__(32 * W, (MT == 2 && !P2POL) ? FG_ROLLOUT_MT2_MIN_BLOCKS : 1) rollout_mma_kernel(const RolloutParams rp) {
+template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL = false>
+__global__ void __launch_bounds__(32 * W, (MT == 2 && !P2POL) ? FG_ROLLOUT_MT2_MIN_BLOCKS : 1)
+rollout_mma_kernel(const typename RolloutArgs<POOL>::type rp) {
     using SM = RolloutMmaSmem<H, W, P2POL>;
     constexpr bool kP2Bot = !P2POL;
     constexpr int kWarpEnvs = 16 * MT, kEnvs = kWarpEnvs * W;
+    static_assert(!POOL || (P2POL && FG_POOL_BLOCK % kEnvs == 0), "a pool CTA plays against one member");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Tables &Tw = *reinterpret_cast<Tables *>(smem_raw + SM::kTables);
     const Tables &T = Tw;
@@ -231,7 +271,11 @@ __global__ void __launch_bounds__(32 * W, (MT == 2 && !P2POL) ? FG_ROLLOUT_MT2_M
 
     load_tables(&Tw, p.tables);
     policy_mma_stage<H>(pw, rp.w, tid, 32 * W);
-    if (P2POL) policy_mma_stage<H>(pw2, rp.w_p2, tid, 32 * W);
+    int member = 0;
+    if constexpr (POOL) {
+        member = pool_member(rp.pool, (long long)blockIdx.x * kEnvs);
+        policy_mma_stage<H>(pw2, pool_weights(rp.pool, member), tid, 32 * W);
+    } else if (P2POL) policy_mma_stage<H>(pw2, rp.w_p2, tid, 32 * W);
     if (tid < FG_STAT_COUNT) s_stats[tid] = 0ull;
     Env e;
     if (valid) load_env<kP2Bot>(p, i, e);
@@ -334,34 +378,42 @@ __global__ void __launch_bounds__(32 * W, (MT == 2 && !P2POL) ? FG_ROLLOUT_MT2_M
     flush_stats(acc, s_stats, lane);
     __syncthreads();
     if (tid < FG_STAT_COUNT && s_stats[tid]) atomicAdd(&p.stats[tid], s_stats[tid]);
+    if constexpr (POOL) pool_flush(rp.pool, member, s_stats, tid);
 }
 
-template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP>
-static cudaError_t launch_rollout_mma_s(cudaStream_t s, const RolloutParams &rp) {
+// RP = RolloutParams, or RolloutPoolParams for the opponent-pool instantiations (POOL)
+template <class RP> constexpr bool kIsPool = std::is_same<RP, RolloutPoolParams>::value;
+
+template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, class RP>
+static cudaError_t launch_rollout_mma_s(cudaStream_t s, const RP &rp) {
+    constexpr bool POOL = kIsPool<RP>;
     constexpr size_t bytes = RolloutMmaSmem<H, W, P2POL>::kBytes;
     static fg::DeviceOnceFlags configured;
     if (cudaError_t e = fg::configure_once_per_device(configured, [] {
-            return cudaFuncSetAttribute(rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
+            return cudaFuncSetAttribute(rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
         return e;
     constexpr int kEnvs = 16 * MT * W;
     const int grid = (rp.sim.n + kEnvs - 1) / kEnvs;
-    rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP><<<grid, 32 * W, bytes, s>>>(rp);
+    rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL><<<grid, 32 * W, bytes, s>>>(rp);
     return cudaSuccess;
 }
-template <int H, int W, bool DENSE>
-static cudaError_t launch_rollout_mma_w(int mt, cudaStream_t s, const RolloutParams &rp) {
+template <int H, int W, bool DENSE, class RP>
+static cudaError_t launch_rollout_mma_w(int mt, cudaStream_t s, const RP &rp) {
     const bool skip = rp.sim.skip_unactionable != 0;
 #define FG_MMA_GO(MT, P2, SK) launch_rollout_mma_s<H, W, MT, DENSE, P2, SK>(s, rp)
-    if (rp.p2_policy) {
+    if (kIsPool<RP> || rp.p2_policy) {
         if (mt == 1) return skip ? FG_MMA_GO(1, true, true) : FG_MMA_GO(1, true, false);
         return skip ? FG_MMA_GO(2, true, true) : FG_MMA_GO(2, true, false);
     }
-    if (mt == 1) return skip ? FG_MMA_GO(1, false, true) : FG_MMA_GO(1, false, false);
-    return skip ? FG_MMA_GO(2, false, true) : FG_MMA_GO(2, false, false);
+    if constexpr (!kIsPool<RP>) {
+        if (mt == 1) return skip ? FG_MMA_GO(1, false, true) : FG_MMA_GO(1, false, false);
+        return skip ? FG_MMA_GO(2, false, true) : FG_MMA_GO(2, false, false);
+    }
 #undef FG_MMA_GO
+    return cudaErrorInvalidValue;
 }
-template <int H, bool DENSE>
-static cudaError_t launch_rollout_mma(cudaStream_t s, const RolloutParams &rp) {
+template <int H, bool DENSE, class RP>
+static cudaError_t launch_rollout_mma(cudaStream_t s, const RP &rp) {
     // Measured (profiles/r02f_rollout_mma.log, H = 64, us per step, 16-battle / 32-battle warps / round-1 FFMA2 kernel):
     // 16 384 battles 4.49 / 5.90 / 6.37; 131 072: 28.0 / 31.3 / -; 1 Mi: 216 / 227 / 262 -- more, lighter warps hide the
     // simulator's latency under the neighbours' tensor-core phases at every size, so 16-battle warps are the default
@@ -378,25 +430,26 @@ static cudaError_t launch_rollout_mma(cudaStream_t s, const RolloutParams &rp) {
     return launch_rollout_mma_w<H, 4, DENSE>(mt, s, rp);
 }
 
-template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP>
-static cudaError_t launch_rollout_s(cudaStream_t s, const RolloutParams &rp) {
+template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, class RP>
+static cudaError_t launch_rollout_s(cudaStream_t s, const RP &rp) {
+    constexpr bool POOL = kIsPool<RP>;
     constexpr size_t bytes = RolloutSmem<H, E, W, P2POL>::kBytes;
     static fg::DeviceOnceFlags configured;
     if (cudaError_t e = fg::configure_once_per_device(configured, [] {
-            return cudaFuncSetAttribute(rollout_kernel<H, E, W, DENSE, P2POL, SKIP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
+            return cudaFuncSetAttribute(rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
         return e;
     constexpr int kEnvs = RolloutSmem<H, E, W, P2POL>::kEnvs;
     const int grid = (rp.sim.n + kEnvs - 1) / kEnvs;
-    rollout_kernel<H, E, W, DENSE, P2POL, SKIP><<<grid, 32 * W, bytes, s>>>(rp);
+    rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL><<<grid, 32 * W, bytes, s>>>(rp);
     return cudaSuccess;
 }
-template <int H, int E, int W, bool DENSE, bool P2POL>
-static cudaError_t launch_rollout_v(cudaStream_t s, const RolloutParams &rp) {
+template <int H, int E, int W, bool DENSE, bool P2POL, class RP>
+static cudaError_t launch_rollout_v(cudaStream_t s, const RP &rp) {
     return rp.sim.skip_unactionable ? launch_rollout_s<H, E, W, DENSE, P2POL, true>(s, rp) : launch_rollout_s<H, E, W, DENSE, P2POL, false>(s, rp);
 }
 
-template <int H, bool DENSE>
-static cudaError_t launch_rollout_h(cudaStream_t s, const RolloutParams &rp) {
+template <int H, bool DENSE, class RP>
+static cudaError_t launch_rollout_h(cudaStream_t s, const RP &rp) {
     if constexpr (H <= kMmaMaxHidden) {
         if (!getenv("FOOTSIES_B200_ROLLOUT_FFMA")) return launch_rollout_mma<H, DENSE>(s, rp);   // knob: the round-1 FFMA2 kernel for A/B runs
     }
@@ -405,18 +458,25 @@ static cudaError_t launch_rollout_h(cudaStream_t s, const RolloutParams &rp) {
     int e = rp.sim.n >= 65536 ? 4 : 2;
     if (const char *v = getenv("FOOTSIES_B200_ROLLOUT_E")) e = atoi(v);   // developer knob
     constexpr int E4 = H <= 64 ? 4 : 2;                                  // H = 128: 4 battles per lane do not fit the registers
-    if (rp.p2_policy)       // two weight sets in shared memory: always 2 battles per lane
+    if (kIsPool<RP> || rp.p2_policy)       // two weight sets in shared memory: always 2 battles per lane
         return launch_rollout_v<H, 2, kPolicyWarps, DENSE, true>(s, rp);
-    if (e == 1) return launch_rollout_v<H, 1, kPolicyWarps, DENSE, false>(s, rp);
-    return e == 4 ? launch_rollout_v<H, E4, kPolicyWarps, DENSE, false>(s, rp) : launch_rollout_v<H, 2, kPolicyWarps, DENSE, false>(s, rp);
+    if constexpr (!kIsPool<RP>) {
+        if (e == 1) return launch_rollout_v<H, 1, kPolicyWarps, DENSE, false>(s, rp);
+        return e == 4 ? launch_rollout_v<H, E4, kPolicyWarps, DENSE, false>(s, rp) : launch_rollout_v<H, 2, kPolicyWarps, DENSE, false>(s, rp);
+    }
+    return cudaErrorInvalidValue;
 }
 
 // One translation unit per hidden size and reward mode (build.py compiles this file with -DFG_ROLLOUT_H=.. -DFG_ROLLOUT_DENSE=..
 // so that the kernels compile in parallel) plus one without the defines that holds the dispatcher.
 #define FG_ROLLOUT_DECL(H, D) cudaError_t launch_rollout_##H##_##D(cudaStream_t s, const RolloutParams &rp)
 FG_ROLLOUT_DECL(32, 0); FG_ROLLOUT_DECL(32, 1); FG_ROLLOUT_DECL(64, 0); FG_ROLLOUT_DECL(64, 1); FG_ROLLOUT_DECL(128, 0); FG_ROLLOUT_DECL(128, 1);
+#define FG_ROLLOUT_POOL_DECL(H, D) cudaError_t launch_rollout_pool_##H##_##D(cudaStream_t s, const RolloutPoolParams &rp)
+FG_ROLLOUT_POOL_DECL(32, 0); FG_ROLLOUT_POOL_DECL(32, 1); FG_ROLLOUT_POOL_DECL(64, 0); FG_ROLLOUT_POOL_DECL(64, 1);
+FG_ROLLOUT_POOL_DECL(128, 0); FG_ROLLOUT_POOL_DECL(128, 1);
 #ifdef FG_ROLLOUT_H
-#define FG_ROLLOUT_DEF2(H, D) FG_ROLLOUT_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); }
+#define FG_ROLLOUT_DEF2(H, D) FG_ROLLOUT_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); } \
+    FG_ROLLOUT_POOL_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); }
 #define FG_ROLLOUT_DEF(H, D) FG_ROLLOUT_DEF2(H, D)
 FG_ROLLOUT_DEF(FG_ROLLOUT_H, FG_ROLLOUT_DENSE)
 #else
@@ -425,6 +485,14 @@ cudaError_t launch_rollout(bool dense, cudaStream_t s, const RolloutParams &rp) 
     case 32: return dense ? launch_rollout_32_1(s, rp) : launch_rollout_32_0(s, rp);
     case 64: return dense ? launch_rollout_64_1(s, rp) : launch_rollout_64_0(s, rp);
     case 128: return dense ? launch_rollout_128_1(s, rp) : launch_rollout_128_0(s, rp);
+    default: return cudaErrorInvalidValue;
+    }
+}
+cudaError_t launch_rollout_pool(bool dense, cudaStream_t s, const RolloutPoolParams &rp) {
+    switch (rp.hidden) {
+    case 32: return dense ? launch_rollout_pool_32_1(s, rp) : launch_rollout_pool_32_0(s, rp);
+    case 64: return dense ? launch_rollout_pool_64_1(s, rp) : launch_rollout_pool_64_0(s, rp);
+    case 128: return dense ? launch_rollout_pool_128_1(s, rp) : launch_rollout_pool_128_0(s, rp);
     default: return cudaErrorInvalidValue;
     }
 }

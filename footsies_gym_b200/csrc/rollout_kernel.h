@@ -26,9 +26,25 @@ struct RolloutParams {
     float *logp_p2;             // [horizon][n]
 };
 
+// P2 from an opponent pool (fg_rollout_mlp_pool): member m plays the battles [end[m - 1], end[m]).  The boundaries are
+// multiples of FG_POOL_BLOCK (or n), so each CTA belongs to one member, stages its weights where the single P2 policy's go
+// and adds its episode results to stats[member][0..3] (optional) when it flushes its statistics at the end.  A separate
+// parameter struct, so that the kernels of the other modes keep their parameters and their code.
+struct RolloutPool {
+    fgp::PolicyWeights member[FG_POOL_MAX];
+    long long end[FG_POOL_MAX];
+    int count;
+    unsigned long long *stats;  // [count][4] or null
+};
+struct RolloutPoolParams : RolloutParams {
+    RolloutPool pool;
+};
+
 // P1 = the MLP policy, P2 = the in-game BattleAI or a second MLP policy (p2_policy), autoreset on.  Returns
 // cudaErrorInvalidValue for other hidden sizes.
 cudaError_t launch_rollout(bool dense, cudaStream_t s, const RolloutParams &rp);
+// The same with P2 from an opponent pool (rp.p2_policy = 1; w_p2 is not read).
+cudaError_t launch_rollout_pool(bool dense, cudaStream_t s, const RolloutPoolParams &rp);
 
 }  // namespace fgk
 #endif

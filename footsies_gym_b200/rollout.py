@@ -13,7 +13,8 @@ Three policy paths:
   * `MLPPolicy`, fused="horizon" (the default whenever the env qualifies: P1 = policy, P2 = in-game bot or a second
     MLPPolicy given as `opponent_policy` (self-play), autoreset, no step mask): ONE launch per horizon (csrc/rollout_kernel.cu, fg_rollout_mlp) -- a CTA keeps its 64 battles in
     registers from the first step to the last and alternates policy inference and the frame update; bit-identical
-    to the per-step path.
+    to the per-step path.  Self-play against an opponent pool (`opponent_pool=[...]`: up to 16 P2 networks, each on its
+    own range of battles, with results per member) runs on this path only (fg_rollout_mlp_pool).
 
 With a value network (`value=`), collect() also returns what a PPO update consumes besides the rollout itself: the values
 of all horizon + 1 observation rows (one fg_value_mlp launch for an `MLPValue` with hidden 32 / 64, else one call of the
@@ -22,7 +23,8 @@ torch callable) and GAE advantages / returns (one fg_gae launch), after the roll
 PyTorch is plumbing here (parameters, buffers, CUDA graph); the simulator step inside the loop is fg_step.
 """
 import ctypes as C
-from typing import Callable, Optional
+import math
+from typing import Callable, List, Optional, Sequence, Tuple
 
 import torch
 
@@ -185,18 +187,58 @@ _MIRROR_ACTION = (0, 2, 1, 3, 4, 6, 5, 7)      # Left (1) <-> Right (2)
 _P2_SEED_SALT = 0x5DEECE66D2F1A3B7
 
 
+def opponent_ranges(num_envs: int, shares: Sequence[float]) -> List[Tuple[int, int]]:
+    """Contiguous battle ranges [(start, end), ...], one per opponent-pool member, in proportion to non-negative `shares`.
+
+    The num_envs // 128 whole blocks of FG_POOL_BLOCK = 128 battles are divided by largest remainder (ties go to the lower
+    index); the battles left over after the last whole block go to the last member with a non-zero share, so that every
+    boundary but the final num_envs is a multiple of 128 -- what fg_rollout_mlp_pool asks of fg_opponent_pool.end.  A member
+    with share 0 gets an empty range.  The ranges cover 0 .. num_envs exactly once, in member order."""
+    shares = [float(s) for s in shares]
+    if not 1 <= len(shares) <= _capi.FG_POOL_MAX:
+        raise ValueError(f"an opponent pool has 1 .. {_capi.FG_POOL_MAX} members (got {len(shares)})")
+    if any(not math.isfinite(s) or s < 0 for s in shares) or sum(shares) <= 0:
+        raise ValueError("opponent shares must be finite, non-negative and not all zero")
+    if num_envs < 1:
+        raise ValueError("num_envs must be positive")
+    block = _capi.FG_POOL_BLOCK
+    blocks = num_envs // block
+    total = sum(shares)
+    quota = [s / total * blocks for s in shares]
+    count = [int(math.floor(q)) for q in quota]
+    order = sorted((i for i in range(len(shares)) if shares[i] > 0), key=lambda i: (-(quota[i] - count[i]), i))
+    for k in range(blocks - sum(count)):
+        count[order[k % len(order)]] += 1
+    last = max(i for i, s in enumerate(shares) if s > 0)
+    ranges, start = [], 0
+    for i, c in enumerate(count):
+        end = num_envs if i >= last else start + c * block
+        ranges.append((start, end))
+        start = end
+    return ranges
+
+
 class RolloutCollector:
     """Collects `horizon` steps of (obs, action, log-prob, reward, done) for every env of one GPU, entirely on device.
 
     Buffers (overwritten by every collect()): obs [horizon + 1, N, 8] (obs[t] is what the policy saw at step t, obs[-1]
     the observation after the last step), actions uint8 [horizon, N], logp / rewards float32 [horizon, N], dones bool;
     with a value network also values float32 [horizon + 1, N] (of every obs row) and advantages / returns float32
-    [horizon, N] (GAE with gamma, gae_lambda; see compute_gae)."""
+    [horizon, N] (GAE with gamma, gae_lambda; see compute_gae).
+
+    Opponent pool (`opponent_pool=[p2_0, p2_1, ...]`, self-play): P2 is played by up to 16 MLPPolicy networks at once, each
+    on its own contiguous range of battles (`opponent_ranges`, set by assign_opponents), in the one launch per horizon of
+    fg_rollout_mlp_pool.  A battle of member m's range draws exactly what it would draw against member m alone.  Results per
+    member accumulate in opponent_pool_stats().  Members are ordinary modules, read at every collect(): a snapshot loaded
+    with load_state_dict is played from the next collect() on, and the live `policy` may itself be a member.  Ranges only
+    change between horizons, but a battle does not restart when they do: a battle re-assigned in mid-episode finishes that
+    episode against its new member, and the result counts for the new member."""
 
     def __init__(self, env: FootsiesEnv, policy: Callable[[torch.Tensor], torch.Tensor], horizon: int = 128,
                  use_cuda_graph: bool = True, fused=None, seed: int = 0,
                  opponent_policy: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, mirror_opponent: bool = False,
-                 value: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, gamma: float = 0.99, gae_lambda: float = 0.95):
+                 value: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, gamma: float = 0.99, gae_lambda: float = 0.95,
+                 opponent_pool: Optional[Sequence["MLPPolicy"]] = None):
         """fused: None / True = the most fused path available ("horizon", else "step", else torch ops for a policy that
         is not an MLPPolicy); False = torch ops; "step" / "horizon" = that path or an error.
         opponent_policy: a second policy for P2 (self-play rollouts; the env must take P2's actions from step(), i.e.
@@ -204,7 +246,12 @@ class RolloutCollector:
         callable (footsies.py:522-527), or its mirror image with mirror_opponent=True (then `policy` itself can be passed
         again: one network plays both sides).  Its actions / log-probabilities are collected in actions_p2 / logp_p2.
         value: a value network, `value(obs[M, 8]) -> [M]` or `[M, 1]`; an MLPValue with hidden 32 / 64 runs on the fused
-        kernel (fg_value_mlp).  The policy path is chosen as without it.  Values and advantages are P1's."""
+        kernel (fg_value_mlp).  The policy path is chosen as without it.  Values and advantages are P1's.
+        opponent_pool: instead of opponent_policy, a list of 1 .. 16 MLPPolicy networks with `policy`'s hidden size that
+        play P2 on separate ranges of battles (see the class docstring; equal shares until assign_opponents is called),
+        each on the mirrored observation with mirror_opponent=True.  Needs an MLPPolicy `policy`, a self-play env with
+        autoreset and no step mask: the whole-horizon kernel (fused=None / True / "horizon"); anything else is a
+        ValueError."""
         if env.by_example:
             raise ValueError("the policy drives P1: create the env with by_example=False")
         if env.frame_delay:
@@ -213,11 +260,14 @@ class RolloutCollector:
         self.opponent_policy, self.mirror_opponent = opponent_policy, bool(mirror_opponent)
         if opponent_policy is not None and (env._opponent_mode == "bot" or env.opponent is not None):
             raise ValueError("opponent_policy needs an env whose P2 actions come from step(): opponent='self_play'")
+        self.opponent_pool = None if opponent_pool is None else list(opponent_pool)
+        if self.opponent_pool is not None:
+            self._check_pool(fused)
         can_step = isinstance(policy, MLPPolicy) and policy.hidden in (32, 64, 128)
         if opponent_policy is not None:
             can_step = can_step and isinstance(opponent_policy, MLPPolicy) and opponent_policy.hidden == policy.hidden
         can_horizon = (can_step and env.autoreset and env._step_mask is None
-                       and (env._opponent_mode == "bot" or opponent_policy is not None))
+                       and (env._opponent_mode == "bot" or opponent_policy is not None or self.opponent_pool is not None))
         if fused is None or fused is True:
             if fused and not can_step:
                 raise ValueError("fused=True needs an MLPPolicy with hidden in {32, 64, 128}")
@@ -238,10 +288,14 @@ class RolloutCollector:
         self.rewards = torch.zeros((h, n), dtype=torch.float32, device=dev)
         self.dones = torch.zeros((h, n), dtype=torch.bool, device=dev)
         self.actions_p2 = self.logp_p2 = None
-        if opponent_policy is not None:
+        if opponent_policy is not None or self.opponent_pool is not None:
             self.actions_p2 = torch.zeros((h, n), dtype=torch.uint8, device=dev)
             self.logp_p2 = torch.zeros((h, n), dtype=torch.float32, device=dev)
             self._mirror_action = torch.tensor(_MIRROR_ACTION, dtype=torch.uint8, device=dev)
+        self.opponent_ranges = None
+        if self.opponent_pool is not None:
+            self._pool_stats = torch.zeros((len(self.opponent_pool), 4), dtype=torch.int64, device=dev)
+            self.assign_opponents()
         self.value, self.gamma, self.gae_lambda = value, float(gamma), float(gae_lambda)
         self.values = self.advantages = self.returns = None
         if value is not None:
@@ -257,8 +311,60 @@ class RolloutCollector:
             env.reset()
         self.obs[h].copy_(env.obs)                                  # the observation the first step will act on
 
+    def _check_pool(self, fused):
+        env, pool = self.env, self.opponent_pool
+        if self.opponent_policy is not None:
+            raise ValueError("opponent_policy and opponent_pool are mutually exclusive")
+        if env._opponent_mode == "bot" or env.opponent is not None:
+            raise ValueError("opponent_pool needs an env whose P2 actions come from step(): opponent='self_play'")
+        if not 1 <= len(pool) <= _capi.FG_POOL_MAX:
+            raise ValueError(f"opponent_pool has 1 .. {_capi.FG_POOL_MAX} members (got {len(pool)})")
+        if not (isinstance(self.policy, MLPPolicy) and self.policy.hidden in (32, 64, 128)):
+            raise ValueError("opponent_pool needs an MLPPolicy with hidden in {32, 64, 128} as the policy")
+        for k, m in enumerate(pool):
+            if not isinstance(m, MLPPolicy) or m.hidden != self.policy.hidden:
+                raise ValueError(f"opponent_pool[{k}] must be an MLPPolicy with the policy's hidden size {self.policy.hidden}")
+        if not env.autoreset or env._step_mask is not None:
+            raise ValueError("opponent_pool runs on the whole-horizon kernel only: the env needs autoreset and no step mask")
+        if fused not in (None, True, "horizon"):
+            raise ValueError("opponent_pool runs on the whole-horizon kernel only: fused must be None, True or 'horizon'")
+
+    def assign_opponents(self, shares: Optional[Sequence[float]] = None):
+        """Splits this device's battles between the pool members in proportion to non-negative `shares` (default: equal),
+        as contiguous block-aligned ranges (see opponent_ranges), from the next collect() on.  Returns the ranges, which
+        are also kept in self.opponent_ranges."""
+        if self.opponent_pool is None:
+            raise ValueError("assign_opponents needs a collector with an opponent_pool")
+        if shares is None:
+            shares = [1.0] * len(self.opponent_pool)
+        if len(shares) != len(self.opponent_pool):
+            raise ValueError(f"one share per pool member: {len(self.opponent_pool)} expected, got {len(shares)}")
+        self.opponent_ranges = opponent_ranges(self.env.num_envs, shares)
+        return self.opponent_ranges
+
+    def opponent_pool_stats(self) -> torch.Tensor:
+        """int64 [K, 4] on the device: episodes, P1 wins, P2 wins, double KOs of the battles each pool member has played,
+        accumulated over every collect() so far (a copy)."""
+        if self.opponent_pool is None:
+            raise ValueError("opponent_pool_stats needs a collector with an opponent_pool")
+        return self._pool_stats.clone()
+
+    def _pool_struct(self):
+        pool = _capi.FgOpponentPool(struct_size=C.sizeof(_capi.FgOpponentPool), count=len(self.opponent_pool),
+                                    stats=self._pool_stats.data_ptr())
+        for k, m in enumerate(self.opponent_pool):
+            l1, l2, l3 = m.net[0], m.net[2], m.net[4]
+            for name, t in dict(scale=m.scale, w1=l1.weight, b1=l1.bias, w2=l2.weight, b2=l2.bias, w3=l3.weight,
+                                b3=l3.bias).items():
+                if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.env.device:
+                    raise ValueError(f"opponent_pool[{k}].{name} must be a contiguous float32 tensor on the env's device")
+                setattr(pool.member[k], name, t.data_ptr())
+            pool.end[k] = self.opponent_ranges[k][1]
+        return pool
+
     def _horizon_launch(self):
-        """fg_rollout_mlp: the whole horizon in one launch on the current stream."""
+        """fg_rollout_mlp (fg_rollout_mlp_pool with an opponent pool): the whole horizon in one launch on the current
+        stream."""
         env, pol = self.env, self.policy
         l1, l2, l3 = pol.net[0], pol.net[2], pol.net[4]
         r = _capi.FgRolloutBuffers(struct_size=C.sizeof(_capi.FgRolloutBuffers), hidden=pol.hidden, horizon=self.horizon,
@@ -273,11 +379,19 @@ class RolloutCollector:
                       p2_b3=m3.bias, actions_p2=self.actions_p2, logp_p2=self.logp_p2)
             r.p2_seed = (self._seed ^ _P2_SEED_SALT) & (2**64 - 1)
             r.p2_mirror = int(self.mirror_opponent)
+        elif self.opponent_pool is not None:
+            ts.update(actions_p2=self.actions_p2, logp_p2=self.logp_p2)
+            r.p2_seed = (self._seed ^ _P2_SEED_SALT) & (2**64 - 1)
+            r.p2_mirror = int(self.mirror_opponent)
         for k, t in ts.items():
             if not t.is_contiguous() or t.device != env.device:
                 raise ValueError(f"fused rollout needs contiguous tensors on the env's device ({k})")
             setattr(r, k, t.data_ptr())
-        _capi.check(env._lib.fg_rollout_mlp(env._handle, C.byref(r), env._stream()))
+        if self.opponent_pool is not None:
+            pool = self._pool_struct()
+            _capi.check(env._lib.fg_rollout_mlp_pool(env._handle, C.byref(r), C.byref(pool), env._stream()))
+        else:
+            _capi.check(env._lib.fg_rollout_mlp(env._handle, C.byref(r), env._stream()))
         self._drawn.add_(self.horizon)
 
     def _values_and_gae(self):
@@ -350,7 +464,7 @@ class RolloutCollector:
             self._graph.replay()
         out = {"obs": self.obs[:self.horizon], "actions": self.actions, "logp": self.logp, "rewards": self.rewards,
                "dones": self.dones, "last_obs": self.obs[self.horizon]}
-        if self.opponent_policy is not None:
+        if self.actions_p2 is not None:
             out.update(actions_p2=self.actions_p2, logp_p2=self.logp_p2)
         if self.value is not None:
             out.update(values=self.values, advantages=self.advantages, returns=self.returns)

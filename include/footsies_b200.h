@@ -24,7 +24,7 @@ extern "C" {
 
 /* 2 (round 2): fg_env_state.p1_bot_memory, first_env_index argument of fg_policy_mlp_sample[_p2], packed host layout
  * (fg_packed_result, fg_step_host_packed, fg_reset_host_packed, fg_packed_reward_table), fg_host_alloc / fg_host_free.
- * Added since, backward compatible (new entry points only, so still 2): fg_value_mlp, fg_gae. */
+ * Added since, backward compatible (new entry points only, so still 2): fg_value_mlp, fg_gae, fg_rollout_mlp_pool. */
 #define FG_ABI_VERSION 2
 
 typedef enum {
@@ -277,6 +277,31 @@ typedef struct {
     int32_t reserved1;
 } fg_rollout_buffers;
 int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream);
+
+/* Self-play against an opponent pool: fg_rollout_mlp with P2 played by up to FG_POOL_MAX MLP policies at once, one per
+ * contiguous range of battles -- member m plays the local battles [end[m - 1], end[m]) (end[-1] = 0), e.g. the learner
+ * and frozen snapshots of it for fictitious self-play.  The reference has no counterpart; its nearest equivalent is the
+ * per-process `opponent(obs, info)` callable (footsies.py:522-527).
+ *   - end is non-decreasing; every boundary is a multiple of FG_POOL_BLOCK or equal to num_envs, and end[count - 1] =
+ *     num_envs.  Empty ranges are allowed.  (A CTA of the kernel owns 64 or 128 battles, so it never spans two members.)
+ *   - Every member has the learner's hidden size r->hidden; its weights are DEVICE pointers in torch.nn.Linear layout
+ *     (w2 16-byte aligned).  r->p2_scale .. r->p2_b3 are ignored; p2_seed, actions_p2, logp_p2 and p2_mirror keep their
+ *     meaning (the mirror applies to every member).  P2's samples depend on (p2_seed, step, GLOBAL battle index) only, so
+ *     a battle of member m's range draws exactly what it would draw against member m alone.
+ *   - stats (optional, DEVICE, 8-byte aligned, [count][4]): episodes, P1 wins, P2 wins and double KOs of each member's
+ *     battles are ADDED to it, next to the handle's own statistics (which count every battle as before).
+ * Needs p2_bot = 0 and everything fg_rollout_mlp needs.  Results are bit-identical to fg_rollout_mlp run on a handle of
+ * just member m's battles (num_envs = end[m] - end[m - 1], first_env_index shifted by end[m - 1]) with member m as P2. */
+#define FG_POOL_MAX 16
+#define FG_POOL_BLOCK 128
+typedef struct { const float *scale, *w1, *b1, *w2, *b2, *w3, *b3; } fg_mlp_weights;
+typedef struct {
+    int32_t struct_size, count;              /* 1 .. FG_POOL_MAX                                                       */
+    fg_mlp_weights member[FG_POOL_MAX];      /* device pointers, torch.nn.Linear layout                                */
+    int64_t end[FG_POOL_MAX];                /* non-decreasing, see above; empty ranges allowed                         */
+    uint64_t *stats;                         /* optional device [count][4]: episodes, P1 wins, P2 wins, double KOs (accumulated) */
+} fg_opponent_pool;
+int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, void *stream);
 
 /* Critic side of an actor-critic (PPO) rollout, for any source of rollout buffers.  Handle-free like fg_policy_mlp_sample;
  * errors are reported through fg_policy_last_error().  All pointers are DEVICE pointers.
