@@ -2,7 +2,7 @@
 """PPO against the in-game bot, entirely on the GPU (BASELINE.json configs[4] in use).
 
     python examples/ppo_footsies.py [--envs 16384] [--horizon 128] [--iters 40] [--frame-skip 1] [--self-play]
-                                    [--pool K --snapshot-every S]
+                                    [--pool K --snapshot-every S [--bot-share F]]
     torchrun --nproc-per-node 8 examples/ppo_footsies.py          # one process per GPU, gradients all-reduced
 
 Rollouts come from footsies_gym_b200.rollout.RolloutCollector: the fused policy kernel samples actions from the
@@ -18,7 +18,9 @@ With --self-play --pool K the opponent is a pool of K networks sharing the battl
 one launch per horizon): member 0 is the live policy, the other K - 1 slots hold frozen snapshots of it, refreshed one
 slot at a time in round-robin order every S iterations (all start as the initial policy).  Each iteration also prints the
 win rate against every member, from the kernel's per-member counters (all-reduced over the ranks, which use the same
-shares).
+shares).  With --bot-share F (0 < F < 1) the in-game bot joins the pool as member K with a share F of the battles, the K
+networks sharing the rest equally (fg_rollout_mlp_pool_bot, still one launch per horizon): the win rate against the bot
+is read from the bot member's counters, and no separate evaluation rollout is run.
 """
 import argparse
 import os
@@ -51,11 +53,15 @@ def main():
     ap.add_argument("--pool", type=int, default=0, help="with --self-play: play against a pool of this many networks "
                     "(the live policy + K - 1 snapshots)")
     ap.add_argument("--snapshot-every", type=int, default=5, help="iterations between two snapshots into the pool")
+    ap.add_argument("--bot-share", type=float, default=None, help="with --pool: add the in-game bot to the pool with this "
+                    "share of the battles (0 < F < 1); the win rate against it comes from its pool counters")
     a = ap.parse_args()
     if a.pool and not a.self_play:
         ap.error("--pool needs --self-play")
     if a.pool < 0 or a.pool > 16 or a.snapshot_every < 1:
         ap.error("--pool must be in 1 .. 16 and --snapshot-every positive")
+    if a.bot_share is not None and (not a.pool or a.pool > 15 or not 0 < a.bot_share < 1):
+        ap.error("--bot-share needs --pool K with K in 1 .. 15 and a share strictly between 0 and 1")
 
     rank, local_rank, world = env_rank_world()
     dev = torch.device("cuda", local_rank)
@@ -78,19 +84,26 @@ def main():
         for m in pool[1:]:
             m.load_state_dict(policy.state_dict())
             m.requires_grad_(False)
+    bot_member = None
+    if a.bot_share is not None:           # the in-game bot as pool member K: the yardstick is measured in the rollout itself
+        bot_member = a.pool
+        pool = pool + ["bot"]
     col = RolloutCollector(env, policy, horizon=a.horizon, use_cuda_graph=True, seed=rank,
                            opponent_policy=policy if a.self_play and not a.pool else None, mirror_opponent=a.self_play,
                            opponent_pool=pool, value=value, gamma=a.gamma, gae_lambda=a.lam)
+    if bot_member is not None:
+        col.assign_opponents([(1 - a.bot_share) / a.pool] * a.pool + [a.bot_share])
     next_slot = 1
     eval_env = eval_col = None
-    if a.self_play:                       # the yardstick stays the in-game bot
+    if a.self_play and bot_member is None:   # the yardstick stays the in-game bot
         eval_env = make_sharded_env(a.envs * world, frame_skip=a.frame_skip, seed=1)
         eval_col = RolloutCollector(eval_env, policy, horizon=a.horizon, seed=1000 + rank)
     n, h = env.num_envs, a.horizon
-    stat_env = eval_env if a.self_play else env
+    stat_env = eval_env if eval_env is not None else env
     prev = stat_env.episode_stats()
     prev_pool = col.opponent_pool_stats() if pool else None
     t_roll = t_upd = 0.0
+    t_warm = None
     for it in range(a.iters):
         t0 = time.perf_counter()
         out = col.collect()
@@ -134,7 +147,7 @@ def main():
             ft = torch.tensor([frames], dtype=torch.int64, device=dev)
             dist.all_reduce(ft)
             frames = int(ft.item())
-        if a.self_play:
+        if eval_col is not None:
             eval_col.collect()
         st = stat_env.all_reduce_stats()
         ep = st["episodes"] - prev["episodes"]
@@ -149,14 +162,19 @@ def main():
                 dist.all_reduce(d)
             d = d.cpu()
             pool_msg = "  win rate vs pool [" + " ".join(f"{int(w) / max(int(e), 1):.2f}" for e, w in d[:, :2].tolist()) + "]"
+            if bot_member is not None:
+                ep, wins = int(d[bot_member, 0]), int(d[bot_member, 1])
             if (it + 1) % a.snapshot_every == 0 and a.pool > 1:
                 pool[next_slot].load_state_dict(policy.state_dict())     # played from the next collect() on
-                next_slot = next_slot % (a.pool - 1) + 1
+                next_slot = next_slot % (a.pool - 1) + 1       # slots 1 .. K - 1 (the bot's slot K is never overwritten)
         if rank == 0:
             print(f"iter {it:3d}  episodes {ep:8d}  win rate vs bot {wins / max(ep, 1):.3f}  mean reward/step {float(rew.mean()):+.4f}  "
                   f"rollout {frames / (t1 - t0) / 1e6:8.1f} M env-frames/s  update {t2 - t1:.2f} s{pool_msg}", flush=True)
+        if it == 0:
+            t_warm = time.perf_counter()                  # the first iteration includes one-time set-up
     if rank == 0:
-        print(f"total: rollouts {t_roll:.1f} s, updates {t_upd:.1f} s")
+        per_iter = f", {(time.perf_counter() - t_warm) / (a.iters - 1):.4f} s per iteration after the first" if a.iters > 1 else ""
+        print(f"total: rollouts {t_roll:.1f} s, updates {t_upd:.1f} s{per_iter}")
     if world > 1:
         dist.destroy_process_group()
 

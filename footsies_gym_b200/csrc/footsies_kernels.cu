@@ -773,7 +773,9 @@ int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) 
     return FG_OK;
 }
 
-int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, void *stream) {
+// fg_rollout_mlp_pool (bot_member = -1) and fg_rollout_mlp_pool_bot: one validation, one parameter block
+static int32_t rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
+                                bool with_bot, void *stream) {
     if (!pool || pool->struct_size != (int32_t)sizeof(fg_opponent_pool))
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool is null or its struct_size does not match%s");
     if (int rc = check_bound(h)) return rc;
@@ -784,12 +786,15 @@ int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_
     if (h->cfg.p2_bot)
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_pool needs p2_bot = 0: the pool plays P2 (the in-game bot cannot be a member)%s");
     if (pool->count < 1 || pool->count > FG_POOL_MAX) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.count must be in 1..16%s");
+    if (with_bot && (bot_member < 0 || bot_member >= pool->count))
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_pool_bot: bot_member must be in 0 .. fg_opponent_pool.count - 1%s");
     const int64_t n = h->cfg.num_envs;
     for (int m = 0; m < pool->count; m++) {
         const int64_t lo = m ? pool->end[m - 1] : 0, e = pool->end[m];
         if (e < lo || e > n) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end must be non-decreasing and at most num_envs%s");
         if (e % FG_POOL_BLOCK && e != n)
             return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end: every boundary must be a multiple of FG_POOL_BLOCK (128) or num_envs%s");
+        if (with_bot && m == bot_member) continue;                  // the bot's weight pointers are not read
         const fg_mlp_weights &w = pool->member[m];
         if (!w.scale || !w.w1 || !w.b1 || !w.w2 || !w.b2 || !w.w3 || !w.b3)
             return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool: null member weight pointer%s");
@@ -805,7 +810,7 @@ int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers: null pointer (actions_p2 and logp_p2 are required)%s");
     if (((uintptr_t)r->obs & 15u) || ((uintptr_t)r->w2 & 15u)) return fail(FG_ERR_INVALID_ARGUMENT, "obs and w2 must be 16-byte aligned%s");
     CUDA_TRY(cudaSetDevice(h->cfg.device));
-    RolloutPoolParams rp;
+    RolloutPoolBotParams rp;
     rp.sim = make_params(h);
     rp.w = { r->scale, r->w1, r->b1, r->w2, r->b2, r->w3, r->b3 };
     rp.seed = r->seed; rp.counter_base = (const unsigned long long *)r->counter_base;
@@ -822,10 +827,21 @@ int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_
     }
     rp.pool.count = pool->count;
     rp.pool.stats = (unsigned long long *)pool->stats;
-    CUDA_TRY(launch_rollout_pool(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
+    rp.bot_member = with_bot ? bot_member : -1;
+    if (with_bot) CUDA_TRY(launch_rollout_pool_bot(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
+    else CUDA_TRY(launch_rollout_pool(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
     h->launches++;
     CUDA_TRY(cudaGetLastError());
     return FG_OK;
+}
+
+int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, void *stream) {
+    return rollout_mlp_pool(h, r, pool, -1, false, stream);
+}
+
+int32_t fg_rollout_mlp_pool_bot(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
+                                void *stream) {
+    return rollout_mlp_pool(h, r, pool, bot_member, true, stream);
 }
 
 int64_t fg_launch_count(fg_handle *h) { return h ? h->launches : 0; }

@@ -21,6 +21,10 @@
 // stages one member's weights in the single P2 policy's place and runs the same horizon loop; its final statistics flush
 // also lands in that member's counters.  Every range equals a single-opponent rollout of just those battles
 // (tests/test_opponent_pool.py); the POOL = false instantiations are the kernels as they were.
+// With the in-game bot as a member (fg_rollout_mlp_pool_bot, BOTM = true), a CTA of the bot's range branches (CTA-uniformly)
+// into the horizon loop of the P2POL = false kernel: RNG plane loaded and stored, bot queried by reset_env / simulate_frame,
+// no P2 weights and no P2 policy pass; actions_p2 receives the bot's held input at the start of each step, logp_p2 zero.
+// Its battles equal a p2_bot = 1 rollout of the same state (tests/test_opponent_pool_bot.py).
 // Compiled with -fmad=false like the step kernel; the policy arithmetic uses explicit fmaf.
 #include <stdlib.h>
 #include <type_traits>
@@ -45,8 +49,9 @@ struct RolloutSmem {
 };
 
 // ---- opponent pool (fg_rollout_mlp_pool): a CTA's P2 weights are those of the member whose range holds its battles ----
-template <bool POOL> struct RolloutArgs { using type = RolloutParams; };
-template <> struct RolloutArgs<true> { using type = RolloutPoolParams; };
+template <bool POOL, bool BOTM> struct RolloutArgs { using type = RolloutParams; };
+template <> struct RolloutArgs<true, false> { using type = RolloutPoolParams; };
+template <> struct RolloutArgs<true, true> { using type = RolloutPoolBotParams; };   // BOTM: one member is the in-game bot
 
 // member of the CTA whose first battle is `first`: the number of boundaries end[0 .. count - 2] at or below it (end is
 // non-decreasing and first < n = end[count - 1]).  Unrolled with constant indices so that the parameter arrays are read
@@ -70,14 +75,19 @@ __device__ __forceinline__ void pool_flush(const RolloutPool &pool, int m, const
     if (pool.stats && tid < 4 && s_stats[tid]) atomicAdd(&pool.stats[(size_t)m * 4 + tid], s_stats[tid]);
 }
 
-template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL = false>
-__global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutArgs<POOL>::type rp) {
+// One CTA's whole horizon.  BOT (opponent pool with the in-game bot as a member, the CTA in the bot's range): P2 is the
+// bot exactly as in the P2POL = false kernel, in the P2POL shared-memory layout, with no P2 weights staged or policy pass.
+// (tid is read in the kernel itself, where the compiler bounds it by __launch_bounds__.)
+template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL, bool BOT, class RP>
+__device__ __forceinline__ void rollout_cta(const RP &rp, const int tid) {
     using SM = RolloutSmem<H, E, W, P2POL>;
     using PL = typename SM::PL;
-    constexpr bool kP2Bot = !P2POL;                             // P2 = in-game bot (needs the RNG plane) or the second policy
+    constexpr bool kP2Pol = P2POL && !BOT;
+    constexpr bool kP2Bot = !kP2Pol;                            // P2 = in-game bot (needs the RNG plane) or the second policy
     constexpr int kEnvs = SM::kEnvs, kRollThreads = 32 * W;
     static_assert(kEnvs <= kRollThreads, "one simulator thread per battle");
     static_assert(!POOL || (P2POL && FG_POOL_BLOCK % kEnvs == 0), "a pool CTA plays against one member");
+    static_assert(!BOT || POOL, "the bot is a pool member");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Tables &Tw = *reinterpret_cast<Tables *>(smem_raw + SM::kTables);
     const Tables &T = Tw;
@@ -87,7 +97,7 @@ __global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutA
     float4 *obs_s = reinterpret_cast<float4 *>(smem_raw + SM::kObs);
     unsigned long long *s_stats = reinterpret_cast<unsigned long long *>(smem_raw + SM::kStats);
     const Params &p = rp.sim;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     const int n = p.n, horizon = rp.horizon;
     const int base = blockIdx.x * kEnvs;
     const int stid = tid;                                       // simulator thread index = battle within the CTA
@@ -100,7 +110,7 @@ __global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutA
     int member = 0;
     if constexpr (POOL) {
         member = pool_member(rp.pool, base);
-        policy_stage_bcast<H, kEnvs, W>(pw2, pool_weights(rp.pool, member), tid, kRollThreads);
+        if (!BOT) policy_stage_bcast<H, kEnvs, W>(pw2, pool_weights(rp.pool, member), tid, kRollThreads);
     } else if (P2POL) policy_stage_bcast<H, kEnvs, W>(pw2, rp.w_p2, tid, kRollThreads);
     if (tid < FG_STAT_COUNT) s_stats[tid] = 0ull;
     Env e;
@@ -141,7 +151,11 @@ __global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutA
             rp.actions[(size_t)t * n + i] = (uint8_t)in1;
             rp.logp[(size_t)t * n + i] = lp;
         }
-        if (P2POL) {
+        if (BOT && valid) {                                     // the bot's input held when the step begins; no log-probability
+            rp.actions_p2[(size_t)t * n + i] = (uint8_t)((e.misc >> FGM_ACTOR2_SHIFT) & 7u);
+            rp.logp_p2[(size_t)t * n + i] = 0.0f;
+        }
+        if (kP2Pol) {
             // the second policy on the same observation rows (mirrored if asked): the sampling threads above have read
             // P1's partial sums before they arrive at the barriers in here, so the activation buffers can be reused
             float x[E][8];
@@ -225,6 +239,18 @@ __global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutA
     if constexpr (POOL) pool_flush(rp.pool, member, s_stats, tid);
 }
 
+template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL = false, bool BOTM = false>
+__global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutArgs<POOL, BOTM>::type rp) {
+    const int tid = threadIdx.x;
+    if constexpr (BOTM) {                                       // CTA-uniform: a CTA's battles belong to one member
+        if (pool_member(rp.pool, (long long)blockIdx.x * RolloutSmem<H, E, W, P2POL>::kEnvs) == rp.bot_member) {
+            rollout_cta<H, E, W, DENSE, P2POL, SKIP, POOL, true>(rp, tid);
+            return;
+        }
+    }
+    rollout_cta<H, E, W, DENSE, P2POL, SKIP, POOL, false>(rp, tid);
+}
+
 // ---- tensor-core version (H <= 64): every WARP owns 16 MT battles for the whole horizon -- policy (policy_mma.cuh: mma.sync
 // m16n8k8 with the 3 x TF32 split, activations never leave the registers between layers) and simulator alike -- so the
 // horizon loop contains no CTA barrier at all: warps drift apart and one warp's simulator phase overlaps its neighbours'
@@ -248,13 +274,15 @@ struct RolloutMmaSmem {
 #ifndef FG_ROLLOUT_MT2_MIN_BLOCKS
 #define FG_ROLLOUT_MT2_MIN_BLOCKS 1
 #endif
-template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL = false>
-__global__ void __launch_bounds__(32 * W, (MT == 2 && !P2POL) ? FG_ROLLOUT_MT2_MIN_BLOCKS : 1)
-rollout_mma_kernel(const typename RolloutArgs<POOL>::type rp) {
+// One CTA's whole horizon; BOT as in rollout_cta.
+template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL, bool BOT, class RP>
+__device__ __forceinline__ void rollout_mma_cta(const RP &rp, const int tid) {
     using SM = RolloutMmaSmem<H, W, P2POL>;
-    constexpr bool kP2Bot = !P2POL;
+    constexpr bool kP2Pol = P2POL && !BOT;
+    constexpr bool kP2Bot = !kP2Pol;
     constexpr int kWarpEnvs = 16 * MT, kEnvs = kWarpEnvs * W;
     static_assert(!POOL || (P2POL && FG_POOL_BLOCK % kEnvs == 0), "a pool CTA plays against one member");
+    static_assert(!BOT || POOL, "the bot is a pool member");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Tables &Tw = *reinterpret_cast<Tables *>(smem_raw + SM::kTables);
     const Tables &T = Tw;
@@ -262,7 +290,7 @@ rollout_mma_kernel(const typename RolloutArgs<POOL>::type rp) {
     float *pw2 = reinterpret_cast<float *>(smem_raw + SM::kPolicy2);
     unsigned long long *s_stats = reinterpret_cast<unsigned long long *>(smem_raw + SM::kStats);
     const Params &p = rp.sim;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     float *obs_w = reinterpret_cast<float *>(smem_raw + SM::kObs) + warp * 256;      // this warp's observation rows
     float *lg_w = reinterpret_cast<float *>(smem_raw + SM::kLogits) + warp * 256;    // ... and logits
     const int n = p.n, horizon = rp.horizon;
@@ -274,7 +302,7 @@ rollout_mma_kernel(const typename RolloutArgs<POOL>::type rp) {
     int member = 0;
     if constexpr (POOL) {
         member = pool_member(rp.pool, (long long)blockIdx.x * kEnvs);
-        policy_mma_stage<H>(pw2, pool_weights(rp.pool, member), tid, 32 * W);
+        if (!BOT) policy_mma_stage<H>(pw2, pool_weights(rp.pool, member), tid, 32 * W);
     } else if (P2POL) policy_mma_stage<H>(pw2, rp.w_p2, tid, 32 * W);
     if (tid < FG_STAT_COUNT) s_stats[tid] = 0ull;
     Env e;
@@ -300,7 +328,7 @@ rollout_mma_kernel(const typename RolloutArgs<POOL>::type rp) {
         // (the random words do not depend on the logits: their 64-bit multiply chains are issued before the MMAs, under
         // whose latency they complete)
         const uint32_t rnd1 = hash3(rp.seed, drawn + (unsigned long long)t, (uint64_t)(p.first_env_index + i));
-        const uint32_t rnd2 = P2POL ? hash3(rp.seed_p2, drawn + (unsigned long long)t, (uint64_t)(p.first_env_index + i)) : 0u;
+        const uint32_t rnd2 = kP2Pol ? hash3(rp.seed_p2, drawn + (unsigned long long)t, (uint64_t)(p.first_env_index + i)) : 0u;
         policy_mma_logits<H, MT, false>(pw, obs_w, lg_w, lane);
         uint32_t in1 = 0u, in2 = 0u;
         if (valid) {
@@ -311,7 +339,11 @@ rollout_mma_kernel(const typename RolloutArgs<POOL>::type rp) {
             rp.actions[(size_t)t * n + i] = (uint8_t)in1;
             rp.logp[(size_t)t * n + i] = lp;
         }
-        if (P2POL) {
+        if (BOT && valid) {                                         // the bot's input held when the step begins; no log-probability
+            rp.actions_p2[(size_t)t * n + i] = (uint8_t)((e.misc >> FGM_ACTOR2_SHIFT) & 7u);
+            rp.logp_p2[(size_t)t * n + i] = 0.0f;
+        }
+        if (kP2Pol) {
             if (rp.p2_mirror) policy_mma_logits<H, MT, true>(pw2, obs_w, lg_w, lane);
             else policy_mma_logits<H, MT, false>(pw2, obs_w, lg_w, lane);
             if (valid) {
@@ -381,20 +413,35 @@ rollout_mma_kernel(const typename RolloutArgs<POOL>::type rp) {
     if constexpr (POOL) pool_flush(rp.pool, member, s_stats, tid);
 }
 
-// RP = RolloutParams, or RolloutPoolParams for the opponent-pool instantiations (POOL)
-template <class RP> constexpr bool kIsPool = std::is_same<RP, RolloutPoolParams>::value;
+template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL = false, bool BOTM = false>
+__global__ void __launch_bounds__(32 * W, (MT == 2 && !P2POL) ? FG_ROLLOUT_MT2_MIN_BLOCKS : 1)
+rollout_mma_kernel(const typename RolloutArgs<POOL, BOTM>::type rp) {
+    const int tid = threadIdx.x;
+    if constexpr (BOTM) {                                           // CTA-uniform: a CTA's battles belong to one member
+        if (pool_member(rp.pool, (long long)blockIdx.x * (16 * MT * W)) == rp.bot_member) {
+            rollout_mma_cta<H, W, MT, DENSE, P2POL, SKIP, POOL, true>(rp, tid);
+            return;
+        }
+    }
+    rollout_mma_cta<H, W, MT, DENSE, P2POL, SKIP, POOL, false>(rp, tid);
+}
+
+// RP = RolloutParams, or RolloutPoolParams for the opponent-pool instantiations (POOL), or RolloutPoolBotParams for those
+// with the in-game bot as a member (POOL and BOTM)
+template <class RP> constexpr bool kIsPoolBot = std::is_same<RP, RolloutPoolBotParams>::value;
+template <class RP> constexpr bool kIsPool = std::is_same<RP, RolloutPoolParams>::value || kIsPoolBot<RP>;
 
 template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, class RP>
 static cudaError_t launch_rollout_mma_s(cudaStream_t s, const RP &rp) {
-    constexpr bool POOL = kIsPool<RP>;
+    constexpr bool POOL = kIsPool<RP>, BOTM = kIsPoolBot<RP>;
     constexpr size_t bytes = RolloutMmaSmem<H, W, P2POL>::kBytes;
     static fg::DeviceOnceFlags configured;
     if (cudaError_t e = fg::configure_once_per_device(configured, [] {
-            return cudaFuncSetAttribute(rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
+            return cudaFuncSetAttribute(rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL, BOTM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
         return e;
     constexpr int kEnvs = 16 * MT * W;
     const int grid = (rp.sim.n + kEnvs - 1) / kEnvs;
-    rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL><<<grid, 32 * W, bytes, s>>>(rp);
+    rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL, BOTM><<<grid, 32 * W, bytes, s>>>(rp);
     return cudaSuccess;
 }
 template <int H, int W, bool DENSE, class RP>
@@ -432,15 +479,15 @@ static cudaError_t launch_rollout_mma(cudaStream_t s, const RP &rp) {
 
 template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, class RP>
 static cudaError_t launch_rollout_s(cudaStream_t s, const RP &rp) {
-    constexpr bool POOL = kIsPool<RP>;
+    constexpr bool POOL = kIsPool<RP>, BOTM = kIsPoolBot<RP>;
     constexpr size_t bytes = RolloutSmem<H, E, W, P2POL>::kBytes;
     static fg::DeviceOnceFlags configured;
     if (cudaError_t e = fg::configure_once_per_device(configured, [] {
-            return cudaFuncSetAttribute(rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
+            return cudaFuncSetAttribute(rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL, BOTM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
         return e;
     constexpr int kEnvs = RolloutSmem<H, E, W, P2POL>::kEnvs;
     const int grid = (rp.sim.n + kEnvs - 1) / kEnvs;
-    rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL><<<grid, 32 * W, bytes, s>>>(rp);
+    rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL, BOTM><<<grid, 32 * W, bytes, s>>>(rp);
     return cudaSuccess;
 }
 template <int H, int E, int W, bool DENSE, bool P2POL, class RP>
@@ -474,9 +521,13 @@ FG_ROLLOUT_DECL(32, 0); FG_ROLLOUT_DECL(32, 1); FG_ROLLOUT_DECL(64, 0); FG_ROLLO
 #define FG_ROLLOUT_POOL_DECL(H, D) cudaError_t launch_rollout_pool_##H##_##D(cudaStream_t s, const RolloutPoolParams &rp)
 FG_ROLLOUT_POOL_DECL(32, 0); FG_ROLLOUT_POOL_DECL(32, 1); FG_ROLLOUT_POOL_DECL(64, 0); FG_ROLLOUT_POOL_DECL(64, 1);
 FG_ROLLOUT_POOL_DECL(128, 0); FG_ROLLOUT_POOL_DECL(128, 1);
+#define FG_ROLLOUT_POOL_BOT_DECL(H, D) cudaError_t launch_rollout_pool_bot_##H##_##D(cudaStream_t s, const RolloutPoolBotParams &rp)
+FG_ROLLOUT_POOL_BOT_DECL(32, 0); FG_ROLLOUT_POOL_BOT_DECL(32, 1); FG_ROLLOUT_POOL_BOT_DECL(64, 0); FG_ROLLOUT_POOL_BOT_DECL(64, 1);
+FG_ROLLOUT_POOL_BOT_DECL(128, 0); FG_ROLLOUT_POOL_BOT_DECL(128, 1);
 #ifdef FG_ROLLOUT_H
 #define FG_ROLLOUT_DEF2(H, D) FG_ROLLOUT_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); } \
-    FG_ROLLOUT_POOL_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); }
+    FG_ROLLOUT_POOL_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); } \
+    FG_ROLLOUT_POOL_BOT_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); }
 #define FG_ROLLOUT_DEF(H, D) FG_ROLLOUT_DEF2(H, D)
 FG_ROLLOUT_DEF(FG_ROLLOUT_H, FG_ROLLOUT_DENSE)
 #else
@@ -493,6 +544,14 @@ cudaError_t launch_rollout_pool(bool dense, cudaStream_t s, const RolloutPoolPar
     case 32: return dense ? launch_rollout_pool_32_1(s, rp) : launch_rollout_pool_32_0(s, rp);
     case 64: return dense ? launch_rollout_pool_64_1(s, rp) : launch_rollout_pool_64_0(s, rp);
     case 128: return dense ? launch_rollout_pool_128_1(s, rp) : launch_rollout_pool_128_0(s, rp);
+    default: return cudaErrorInvalidValue;
+    }
+}
+cudaError_t launch_rollout_pool_bot(bool dense, cudaStream_t s, const RolloutPoolBotParams &rp) {
+    switch (rp.hidden) {
+    case 32: return dense ? launch_rollout_pool_bot_32_1(s, rp) : launch_rollout_pool_bot_32_0(s, rp);
+    case 64: return dense ? launch_rollout_pool_bot_64_1(s, rp) : launch_rollout_pool_bot_64_0(s, rp);
+    case 128: return dense ? launch_rollout_pool_bot_128_1(s, rp) : launch_rollout_pool_bot_128_0(s, rp);
     default: return cudaErrorInvalidValue;
     }
 }

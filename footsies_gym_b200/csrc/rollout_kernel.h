@@ -39,12 +39,19 @@ struct RolloutPool {
 struct RolloutPoolParams : RolloutParams {
     RolloutPool pool;
 };
+// The same with member bot_member played by the in-game BattleAI (fg_rollout_mlp_pool_bot): its CTAs run the P2 = bot
+// horizon loop, and its weight pointers are never read.
+struct RolloutPoolBotParams : RolloutPoolParams {
+    int bot_member;
+};
 
 // P1 = the MLP policy, P2 = the in-game BattleAI or a second MLP policy (p2_policy), autoreset on.  Returns
 // cudaErrorInvalidValue for other hidden sizes.
 cudaError_t launch_rollout(bool dense, cudaStream_t s, const RolloutParams &rp);
 // The same with P2 from an opponent pool (rp.p2_policy = 1; w_p2 is not read).
 cudaError_t launch_rollout_pool(bool dense, cudaStream_t s, const RolloutPoolParams &rp);
+// The same with member rp.bot_member played by the in-game bot (its weights are not read).
+cudaError_t launch_rollout_pool_bot(bool dense, cudaStream_t s, const RolloutPoolBotParams &rp);
 
 }  // namespace fgk
 #endif

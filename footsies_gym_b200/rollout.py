@@ -14,7 +14,8 @@ Three policy paths:
     MLPPolicy given as `opponent_policy` (self-play), autoreset, no step mask): ONE launch per horizon (csrc/rollout_kernel.cu, fg_rollout_mlp) -- a CTA keeps its 64 battles in
     registers from the first step to the last and alternates policy inference and the frame update; bit-identical
     to the per-step path.  Self-play against an opponent pool (`opponent_pool=[...]`: up to 16 P2 networks, each on its
-    own range of battles, with results per member) runs on this path only (fg_rollout_mlp_pool).
+    own range of battles, with results per member) runs on this path only (fg_rollout_mlp_pool); one member may be the
+    in-game bot, "bot" (fg_rollout_mlp_pool_bot).
 
 With a value network (`value=`), collect() also returns what a PPO update consumes besides the rollout itself: the values
 of all horizon + 1 observation rows (one fg_value_mlp launch for an `MLPValue` with hidden 32 / 64, else one call of the
@@ -232,13 +233,21 @@ class RolloutCollector:
     member accumulate in opponent_pool_stats().  Members are ordinary modules, read at every collect(): a snapshot loaded
     with load_state_dict is played from the next collect() on, and the live `policy` may itself be a member.  Ranges only
     change between horizons, but a battle does not restart when they do: a battle re-assigned in mid-episode finishes that
-    episode against its new member, and the result counts for the new member."""
+    episode against its new member, and the result counts for the new member.
+
+    One member may be the string "bot": the in-game BattleAI plays its range, bit for bit as a rollout on an
+    opponent="bot" env holding the same battle state would (fg_rollout_mlp_pool_bot), so that e.g. past snapshots and the
+    scripted opponent share one rollout and the win rate against the bot is a row of opponent_pool_stats().  In its
+    battles actions_p2 holds the bot's input at the start of each step and logp_p2 is 0 (not a log-probability).  A battle
+    moved into the bot's range continues its episode with empty bot queues and P2's last held input; the first round
+    after env.reset() of a battle in the bot's range starts like such an entry (a self-play env's reset does not ask the
+    bot for its Fight-transition input), every later round exactly as on a bot env."""
 
     def __init__(self, env: FootsiesEnv, policy: Callable[[torch.Tensor], torch.Tensor], horizon: int = 128,
                  use_cuda_graph: bool = True, fused=None, seed: int = 0,
                  opponent_policy: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, mirror_opponent: bool = False,
                  value: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, gamma: float = 0.99, gae_lambda: float = 0.95,
-                 opponent_pool: Optional[Sequence["MLPPolicy"]] = None):
+                 opponent_pool: Optional[Sequence] = None):
         """fused: None / True = the most fused path available ("horizon", else "step", else torch ops for a policy that
         is not an MLPPolicy); False = torch ops; "step" / "horizon" = that path or an error.
         opponent_policy: a second policy for P2 (self-play rollouts; the env must take P2's actions from step(), i.e.
@@ -249,9 +258,10 @@ class RolloutCollector:
         kernel (fg_value_mlp).  The policy path is chosen as without it.  Values and advantages are P1's.
         opponent_pool: instead of opponent_policy, a list of 1 .. 16 MLPPolicy networks with `policy`'s hidden size that
         play P2 on separate ranges of battles (see the class docstring; equal shares until assign_opponents is called),
-        each on the mirrored observation with mirror_opponent=True.  Needs an MLPPolicy `policy`, a self-play env with
-        autoreset and no step mask: the whole-horizon kernel (fused=None / True / "horizon"); anything else is a
-        ValueError."""
+        each on the mirrored observation with mirror_opponent=True.  At most one entry may be the string "bot" (the in-game
+        bot, as in FootsiesEnv(opponent="bot")); it counts as a member for shares and statistics, and mirror_opponent does
+        not apply to it.  Needs an MLPPolicy `policy`, a self-play env with autoreset and no step mask: the whole-horizon
+        kernel (fused=None / True / "horizon"); anything else is a ValueError."""
         if env.by_example:
             raise ValueError("the policy drives P1: create the env with by_example=False")
         if env.frame_delay:
@@ -261,6 +271,7 @@ class RolloutCollector:
         if opponent_policy is not None and (env._opponent_mode == "bot" or env.opponent is not None):
             raise ValueError("opponent_policy needs an env whose P2 actions come from step(): opponent='self_play'")
         self.opponent_pool = None if opponent_pool is None else list(opponent_pool)
+        self._pool_bot = None                                       # index of the "bot" member, if any
         if self.opponent_pool is not None:
             self._check_pool(fused)
         can_step = isinstance(policy, MLPPolicy) and policy.hidden in (32, 64, 128)
@@ -321,9 +332,14 @@ class RolloutCollector:
             raise ValueError(f"opponent_pool has 1 .. {_capi.FG_POOL_MAX} members (got {len(pool)})")
         if not (isinstance(self.policy, MLPPolicy) and self.policy.hidden in (32, 64, 128)):
             raise ValueError("opponent_pool needs an MLPPolicy with hidden in {32, 64, 128} as the policy")
+        bots = [k for k, m in enumerate(pool) if isinstance(m, str) and m == "bot"]
+        if len(bots) > 1:
+            raise ValueError(f'opponent_pool may hold the in-game bot ("bot") once (found at {bots})')
+        self._pool_bot = bots[0] if bots else None
         for k, m in enumerate(pool):
-            if not isinstance(m, MLPPolicy) or m.hidden != self.policy.hidden:
-                raise ValueError(f"opponent_pool[{k}] must be an MLPPolicy with the policy's hidden size {self.policy.hidden}")
+            if k != self._pool_bot and (not isinstance(m, MLPPolicy) or m.hidden != self.policy.hidden):
+                raise ValueError(f'opponent_pool[{k}] must be "bot" or an MLPPolicy with the policy\'s hidden size '
+                                 f'{self.policy.hidden}')
         if not env.autoreset or env._step_mask is not None:
             raise ValueError("opponent_pool runs on the whole-horizon kernel only: the env needs autoreset and no step mask")
         if fused not in (None, True, "horizon"):
@@ -353,18 +369,20 @@ class RolloutCollector:
         pool = _capi.FgOpponentPool(struct_size=C.sizeof(_capi.FgOpponentPool), count=len(self.opponent_pool),
                                     stats=self._pool_stats.data_ptr())
         for k, m in enumerate(self.opponent_pool):
+            pool.end[k] = self.opponent_ranges[k][1]
+            if k == self._pool_bot:                                 # the bot's weight pointers stay null
+                continue
             l1, l2, l3 = m.net[0], m.net[2], m.net[4]
             for name, t in dict(scale=m.scale, w1=l1.weight, b1=l1.bias, w2=l2.weight, b2=l2.bias, w3=l3.weight,
                                 b3=l3.bias).items():
                 if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.env.device:
                     raise ValueError(f"opponent_pool[{k}].{name} must be a contiguous float32 tensor on the env's device")
                 setattr(pool.member[k], name, t.data_ptr())
-            pool.end[k] = self.opponent_ranges[k][1]
         return pool
 
     def _horizon_launch(self):
-        """fg_rollout_mlp (fg_rollout_mlp_pool with an opponent pool): the whole horizon in one launch on the current
-        stream."""
+        """fg_rollout_mlp (fg_rollout_mlp_pool with an opponent pool, fg_rollout_mlp_pool_bot when the bot is one of its
+        members): the whole horizon in one launch on the current stream."""
         env, pol = self.env, self.policy
         l1, l2, l3 = pol.net[0], pol.net[2], pol.net[4]
         r = _capi.FgRolloutBuffers(struct_size=C.sizeof(_capi.FgRolloutBuffers), hidden=pol.hidden, horizon=self.horizon,
@@ -389,7 +407,11 @@ class RolloutCollector:
             setattr(r, k, t.data_ptr())
         if self.opponent_pool is not None:
             pool = self._pool_struct()
-            _capi.check(env._lib.fg_rollout_mlp_pool(env._handle, C.byref(r), C.byref(pool), env._stream()))
+            if self._pool_bot is None:
+                _capi.check(env._lib.fg_rollout_mlp_pool(env._handle, C.byref(r), C.byref(pool), env._stream()))
+            else:
+                _capi.check(env._lib.fg_rollout_mlp_pool_bot(env._handle, C.byref(r), C.byref(pool), self._pool_bot,
+                                                             env._stream()))
         else:
             _capi.check(env._lib.fg_rollout_mlp(env._handle, C.byref(r), env._stream()))
         self._drawn.add_(self.horizon)

@@ -24,7 +24,7 @@ extern "C" {
 
 /* 2 (round 2): fg_env_state.p1_bot_memory, first_env_index argument of fg_policy_mlp_sample[_p2], packed host layout
  * (fg_packed_result, fg_step_host_packed, fg_reset_host_packed, fg_packed_reward_table), fg_host_alloc / fg_host_free.
- * Added since, backward compatible (new entry points only, so still 2): fg_value_mlp, fg_gae, fg_rollout_mlp_pool. */
+ * Added since, backward compatible (new entry points only, so still 2): fg_value_mlp, fg_gae, fg_rollout_mlp_pool, fg_rollout_mlp_pool_bot. */
 #define FG_ABI_VERSION 2
 
 typedef enum {
@@ -302,6 +302,24 @@ typedef struct {
     uint64_t *stats;                         /* optional device [count][4]: episodes, P1 wins, P2 wins, double KOs (accumulated) */
 } fg_opponent_pool;
 int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, void *stream);
+
+/* fg_rollout_mlp_pool with the in-game BattleAI as pool member bot_member (0 .. count - 1), e.g. past snapshots plus the
+ * scripted opponent in one rollout, with the win rate against the bot in stats[bot_member].  member[bot_member]'s weight
+ * pointers are ignored and may be null; every other member's are checked as by fg_rollout_mlp_pool.  The handle still
+ * needs p2_bot = 0; the bot draws from the RNG plane that fg_seed wrote, as on a p2_bot = 1 handle.
+ *   - Twin equality: a battle of the bot's range evolves bit for bit as fg_rollout_mlp evolves it on a p2_bot = 1 handle
+ *     holding the same state: the same four state planes (RNG, bot queues and held inputs included), the same carried-
+ *     over observation row (obs[horizon]), the same seed, counter base and first_env_index shift.  Mid-episode too.
+ *   - In the bot's battles actions_p2[t] is the input the bot holds when step t begins (the held-input bits before the
+ *     step; for frame_skip 1 the input of the step's first frame) and logp_p2[t] is 0.0f, which is NOT a log-probability.
+ *   - Ranges change only between calls.  A battle that moves into the bot's range continues its episode with the BattleAI
+ *     state stored in the battle: empty queues since its last reset (every reset clears them, whoever plays P2) and P2's
+ *     last held input for the first frame.  A battle that leaves the bot's range is played by its new member's network.
+ *   - A self-play handle's fg_reset does not query the bot at the Fight transition, so the first round after fg_reset of a
+ *     battle in the bot's range starts like a mid-episode entry.  Every round the kernel resets itself (autoreset) is
+ *     exactly the bot handle's round. */
+int32_t fg_rollout_mlp_pool_bot(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool,
+                                int32_t bot_member, void *stream);
 
 /* Critic side of an actor-critic (PPO) rollout, for any source of rollout buffers.  Handle-free like fg_policy_mlp_sample;
  * errors are reported through fg_policy_last_error().  All pointers are DEVICE pointers.
