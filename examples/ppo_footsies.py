@@ -42,6 +42,8 @@ def main():
     ap.add_argument("--horizon", type=int, default=128)
     ap.add_argument("--iters", type=int, default=40)
     ap.add_argument("--frame-skip", type=int, default=1)
+    ap.add_argument("--frame-delay", type=int, default=0, help="observations delayed by this many steps (the reference's "
+                    "frame_delay, a model of reaction time), in training and evaluation alike")
     ap.add_argument("--epochs", type=int, default=2)
     ap.add_argument("--minibatches", type=int, default=8)
     ap.add_argument("--lr", type=float, default=1e-3)
@@ -70,7 +72,8 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     torch.manual_seed(0)
 
-    env = make_sharded_env(a.envs * world, frame_skip=a.frame_skip, seed=0, opponent="self_play" if a.self_play else None)
+    env = make_sharded_env(a.envs * world, frame_skip=a.frame_skip, frame_delay=a.frame_delay, seed=0,
+                           opponent="self_play" if a.self_play else None)
     policy = MLPPolicy(64).to(dev)
     value = MLPValue(64).to(dev)
     params = list(policy.parameters()) + list(value.parameters())
@@ -96,7 +99,7 @@ def main():
     next_slot = 1
     eval_env = eval_col = None
     if a.self_play and bot_member is None:   # the yardstick stays the in-game bot
-        eval_env = make_sharded_env(a.envs * world, frame_skip=a.frame_skip, seed=1)
+        eval_env = make_sharded_env(a.envs * world, frame_skip=a.frame_skip, frame_delay=a.frame_delay, seed=1)
         eval_col = RolloutCollector(eval_env, policy, horizon=a.horizon, seed=1000 + rank)
     n, h = env.num_envs, a.horizon
     stat_env = eval_env if eval_env is not None else env

@@ -60,6 +60,12 @@ class FgOpponentPool(C.Structure):
                 ("end", C.c_int64 * FG_POOL_MAX), ("stats", C.c_void_p)]
 
 
+class FgDelayRing(C.Structure):
+    _fields_ = [("struct_size", C.c_int32), ("depth", C.c_int32), ("pos", C.c_int32), ("reserved0", C.c_int32),
+                ("ring_obs", C.c_void_p), ("ring_frame", C.c_void_p), ("ring_misc", C.c_void_p),
+                ("out_obs", C.c_void_p), ("out_frame", C.c_void_p), ("out_misc", C.c_void_p)]
+
+
 class FgFighterState(C.Structure):
     _fields_ = [("pos_x", C.c_float), ("velocity_x", C.c_float), ("action_id", C.c_int32),
                 ("action_frame", C.c_int32), ("hitstun", C.c_int32), ("guard", C.c_int32), ("vital", C.c_int32),
@@ -132,7 +138,7 @@ EXPORTS = ["fg_abi_version", "fg_last_error", "fg_algorithmic_bytes_per_env_step
            "fg_reset_host_compact", "fg_packed_reward_table", "fg_step_host_packed", "fg_reset_host_packed", "fg_host_alloc",
            "fg_host_free", "fg_delay_ring_step", "fg_get_state",
            "fg_set_state", "fg_read_stats", "fg_launch_count", "fg_policy_mlp_sample", "fg_policy_mlp_sample_p2", "fg_policy_last_error",
-           "fg_rollout_mlp", "fg_rollout_mlp_pool", "fg_rollout_mlp_pool_bot", "fg_value_mlp", "fg_gae"]
+           "fg_rollout_mlp", "fg_rollout_mlp_pool", "fg_rollout_mlp_pool_bot", "fg_rollout_mlp_delayed", "fg_value_mlp", "fg_gae"]
 
 
 def load(build_if_missing=True):
@@ -205,6 +211,9 @@ def load(build_if_missing=True):
     L.fg_rollout_mlp_pool.argtypes = [vp, C.POINTER(FgRolloutBuffers), C.POINTER(FgOpponentPool), vp]
     L.fg_rollout_mlp_pool_bot.restype = i32
     L.fg_rollout_mlp_pool_bot.argtypes = [vp, C.POINTER(FgRolloutBuffers), C.POINTER(FgOpponentPool), i32, vp]
+    L.fg_rollout_mlp_delayed.restype = i32
+    L.fg_rollout_mlp_delayed.argtypes = [vp, C.POINTER(FgRolloutBuffers), C.POINTER(FgOpponentPool), i32,
+                                         C.POINTER(FgDelayRing), vp]
     L.fg_value_mlp.restype = i32
     L.fg_value_mlp.argtypes = [vp] * 8 + [i32, i64, vp, vp]
     L.fg_gae.restype = i32

@@ -37,7 +37,7 @@ def deps():
     inc = os.path.join(os.path.dirname(PKG_DIR), "include", "footsies_b200.h")
     return sources() + [os.path.join(CSRC, f) for f in ("state_codec.h", "frame_tables.h", "frame_logic.cuh",
                                                         "tables_host.h", "step_kernel.cuh", "policy_mlp.cuh", "policy_mma.cuh", "device_once.h",
-                                                        "rollout_kernel.h")] + [inc]
+                                                        "rollout_kernel.h", "delay_ring.cuh")] + [inc]
 
 
 def source_digest(extra_flags=()):
@@ -81,6 +81,8 @@ def translation_units():
         for dense in (0, 1):
             units.append((f"rollout_h{hidden}_d{dense}.o", os.path.join(CSRC, "rollout_kernel.cu"),
                           [f"-DFG_ROLLOUT_H={hidden}", f"-DFG_ROLLOUT_DENSE={dense}"]))
+            units.append((f"rollout_delay_h{hidden}_d{dense}.o", os.path.join(CSRC, "rollout_kernel.cu"),
+                          [f"-DFG_ROLLOUT_H={hidden}", f"-DFG_ROLLOUT_DENSE={dense}", "-DFG_ROLLOUT_DELAY=1"]))
     for kf in (0, 1):
         for b1 in (0, 1):
             for b2 in (0, 1):

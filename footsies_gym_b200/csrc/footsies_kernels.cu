@@ -4,6 +4,7 @@
 #include <stdlib.h>
 #include <algorithm>
 
+#include "delay_ring.cuh"
 #include "rollout_kernel.h"
 #include "step_kernel.cuh"
 
@@ -144,54 +145,22 @@ __global__ void __launch_bounds__(256) pack_obs_kernel(const float4 *__restrict_
     }
 }
 
-// The frame_delay queue of FootsiesEnv (footsies.py:129-131: deque(maxlen = frame_delay + 1); :533-535: append the newest
-// state, emit the oldest; :502-504: a reset refills the queue with the first state) as a ring of `depth` slots per battle
-// in device memory: one thread per battle writes the state the step kernel just produced into slot `pos` (into every
-// slot when the battle was reset by this step: info frame == -1) and emits slot (pos + 1) % depth.  44 B read + 44 B
-// written + 44 B emitted per battle and step.
+// The frame_delay queue of FootsiesEnv (delay_ring.cuh) after an fg_step: one thread per battle pushes the state the step
+// kernel just produced at ring position `pos` and emits the delayed state to out_*.  44 B read + 44 B written + 44 B
+// emitted per battle and step.
 __global__ void __launch_bounds__(256) delay_ring_kernel(const float4 *__restrict__ obs, const int32_t *__restrict__ frame,
-                                                         const uint32_t *__restrict__ misc, float4 *ring_obs, int32_t *ring_frame,
-                                                         uint32_t *ring_misc, float4 *__restrict__ out_obs, int32_t *__restrict__ out_frame,
+                                                         const uint32_t *__restrict__ misc, DelayRingRef ring,
+                                                         float4 *__restrict__ out_obs, int32_t *__restrict__ out_frame,
                                                          uint32_t *__restrict__ out_misc, const uint8_t *__restrict__ step_mask,
                                                          int n, int depth, int pos) {
-    const int oldest = (pos + 1) % depth;
+    const int oldest = (pos + 1) % depth, newest = (pos + depth - 1) % depth;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const int32_t f_now = frame[i];
-        if ((step_mask && !step_mask[i]) || (f_now != -1 && f_now == ring_frame[(size_t)((pos + depth - 1) % depth) * n + i])) {
-            // a battle that did not advance -- held back by the step mask, or over and waiting for its reset (its frame
-            // counter still is the newest entry's) -- keeps its queue and its last emitted state (the reference's deque is
-            // per env, footsies.py:129-131); the ring position is shared, so its slots move along with it instead
-            const size_t last = (size_t)(depth - 1) * n + i;
-            float4 ca = ring_obs[2 * last], cb = ring_obs[2 * last + 1];
-            int32_t cf = ring_frame[last];
-            uint32_t cm = ring_misc[last];
-            for (int s = 0; s < depth; s++) {
-                const size_t k = (size_t)s * n + i;
-                const float4 ta = ring_obs[2 * k], tb = ring_obs[2 * k + 1];
-                const int32_t tf = ring_frame[k];
-                const uint32_t tm = ring_misc[k];
-                ring_obs[2 * k] = ca; ring_obs[2 * k + 1] = cb; ring_frame[k] = cf; ring_misc[k] = cm;
-                ca = ta; cb = tb; cf = tf; cm = tm;
-            }
-            continue;
+        DelayEntry now, emit;
+        now.a = obs[2 * (size_t)i]; now.b = obs[2 * (size_t)i + 1]; now.frame = frame[i]; now.misc = misc[i];
+        if (delay_ring_push(ring, i, depth, pos, step_mask && !step_mask[i], now, ring.load(oldest, i),
+                            ring.frame[(size_t)newest * n + i], emit)) {
+            out_obs[2 * (size_t)i] = emit.a; out_obs[2 * (size_t)i + 1] = emit.b; out_frame[i] = emit.frame; out_misc[i] = emit.misc;
         }
-        const float4 a = obs[2 * (size_t)i], b = obs[2 * (size_t)i + 1];
-        const int32_t f = frame[i];
-        const uint32_t m = misc[i];
-        float4 oa = a, ob = b;
-        int32_t of = f;
-        uint32_t om = m;
-        if (f == -1) {
-            for (int s = 0; s < depth; s++) {
-                const size_t k = (size_t)s * n + i;
-                ring_obs[2 * k] = a; ring_obs[2 * k + 1] = b; ring_frame[k] = f; ring_misc[k] = m;
-            }
-        } else {
-            const size_t k = (size_t)pos * n + i, o = (size_t)oldest * n + i;
-            ring_obs[2 * k] = a; ring_obs[2 * k + 1] = b; ring_frame[k] = f; ring_misc[k] = m;
-            oa = ring_obs[2 * o]; ob = ring_obs[2 * o + 1]; of = ring_frame[o]; om = ring_misc[o];
-        }
-        out_obs[2 * (size_t)i] = oa; out_obs[2 * (size_t)i + 1] = ob; out_frame[i] = of; out_misc[i] = om;
     }
 }
 
@@ -732,15 +701,17 @@ int32_t fg_delay_ring_step(fg_handle *h, int32_t depth, int32_t pos, float *ring
     if (((uintptr_t)ring_obs & 15u) || ((uintptr_t)out_obs & 15u) || ((uintptr_t)ring_misc & 3u) || ((uintptr_t)out_misc & 3u))
         return fail(FG_ERR_INVALID_ARGUMENT, "obs buffers must be 16-byte, misc buffers 4-byte aligned%s");
     CUDA_TRY(cudaSetDevice(h->cfg.device));
+    const DelayRingRef ring = { (float4 *)ring_obs, ring_frame, (uint32_t *)ring_misc, (size_t)h->cfg.num_envs };
     delay_ring_kernel<<<grid_for(h, 8), 256, 0, (cudaStream_t)stream>>>(
-        (const float4 *)h->buf.obs, h->buf.info_frame, (const uint32_t *)h->buf.info_misc, (float4 *)ring_obs, ring_frame,
-        (uint32_t *)ring_misc, (float4 *)out_obs, out_frame, (uint32_t *)out_misc, h->buf.step_mask, h->cfg.num_envs, depth, pos);
+        (const float4 *)h->buf.obs, h->buf.info_frame, (const uint32_t *)h->buf.info_misc, ring, (float4 *)out_obs, out_frame,
+        (uint32_t *)out_misc, h->buf.step_mask, h->cfg.num_envs, depth, pos);
     h->launches++;
     CUDA_TRY(cudaGetLastError());
     return FG_OK;
 }
 
-int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) {
+// fg_rollout_mlp's checks and parameter block (also the no-pool case of fg_rollout_mlp_delayed)
+static int32_t rollout_mlp_params(fg_handle *h, const fg_rollout_buffers *r, RolloutParams &rp) {
     if (int rc = check_bound(h)) return rc;
     if (!r || r->struct_size != (int32_t)sizeof(fg_rollout_buffers))
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers is null or its struct_size does not match%s");
@@ -757,8 +728,6 @@ int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) 
     if (!r->scale || !r->w1 || !r->b1 || !r->w2 || !r->b2 || !r->w3 || !r->b3 || !r->obs || !r->actions || !r->logp || !r->rewards || !r->dones)
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers: null pointer%s");
     if (((uintptr_t)r->obs & 15u) || ((uintptr_t)r->w2 & 15u)) return fail(FG_ERR_INVALID_ARGUMENT, "obs and w2 must be 16-byte aligned%s");
-    CUDA_TRY(cudaSetDevice(h->cfg.device));
-    RolloutParams rp;
     rp.sim = make_params(h);
     rp.w = { r->scale, r->w1, r->b1, r->w2, r->b2, r->w3, r->b3 };
     rp.seed = r->seed; rp.counter_base = (const unsigned long long *)r->counter_base;
@@ -767,15 +736,22 @@ int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) 
     rp.p2_policy = p2_policy; rp.p2_mirror = p2_policy && r->p2_mirror;
     rp.w_p2 = { r->p2_scale, r->p2_w1, r->p2_b1, r->p2_w2, r->p2_b2, r->p2_w3, r->p2_b3 };
     rp.seed_p2 = r->p2_seed; rp.actions_p2 = r->actions_p2; rp.logp_p2 = r->logp_p2;
+    return FG_OK;
+}
+
+int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) {
+    RolloutParams rp;
+    if (int rc = rollout_mlp_params(h, r, rp)) return rc;
+    CUDA_TRY(cudaSetDevice(h->cfg.device));
     CUDA_TRY(launch_rollout(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
     h->launches++;
     CUDA_TRY(cudaGetLastError());
     return FG_OK;
 }
 
-// fg_rollout_mlp_pool (bot_member = -1) and fg_rollout_mlp_pool_bot: one validation, one parameter block
-static int32_t rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
-                                bool with_bot, void *stream) {
+// fg_rollout_mlp_pool's and fg_rollout_mlp_pool_bot's checks and parameter block (bot_member = -1 without the bot)
+static int32_t rollout_pool_params(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
+                                   bool with_bot, RolloutPoolBotParams &rp) {
     if (!pool || pool->struct_size != (int32_t)sizeof(fg_opponent_pool))
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool is null or its struct_size does not match%s");
     if (int rc = check_bound(h)) return rc;
@@ -809,8 +785,6 @@ static int32_t rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const
         !r->dones || !r->actions_p2 || !r->logp_p2)
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers: null pointer (actions_p2 and logp_p2 are required)%s");
     if (((uintptr_t)r->obs & 15u) || ((uintptr_t)r->w2 & 15u)) return fail(FG_ERR_INVALID_ARGUMENT, "obs and w2 must be 16-byte aligned%s");
-    CUDA_TRY(cudaSetDevice(h->cfg.device));
-    RolloutPoolBotParams rp;
     rp.sim = make_params(h);
     rp.w = { r->scale, r->w1, r->b1, r->w2, r->b2, r->w3, r->b3 };
     rp.seed = r->seed; rp.counter_base = (const unsigned long long *)r->counter_base;
@@ -828,6 +802,15 @@ static int32_t rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const
     rp.pool.count = pool->count;
     rp.pool.stats = (unsigned long long *)pool->stats;
     rp.bot_member = with_bot ? bot_member : -1;
+    return FG_OK;
+}
+
+// fg_rollout_mlp_pool (bot_member = -1) and fg_rollout_mlp_pool_bot
+static int32_t rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
+                                bool with_bot, void *stream) {
+    RolloutPoolBotParams rp;
+    if (int rc = rollout_pool_params(h, r, pool, bot_member, with_bot, rp)) return rc;
+    CUDA_TRY(cudaSetDevice(h->cfg.device));
     if (with_bot) CUDA_TRY(launch_rollout_pool_bot(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
     else CUDA_TRY(launch_rollout_pool(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
     h->launches++;
@@ -842,6 +825,35 @@ int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_
 int32_t fg_rollout_mlp_pool_bot(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
                                 void *stream) {
     return rollout_mlp_pool(h, r, pool, bot_member, true, stream);
+}
+
+int32_t fg_rollout_mlp_delayed(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
+                               const fg_delay_ring *ring, void *stream) {
+    if (!ring || ring->struct_size != (int32_t)sizeof(fg_delay_ring))
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_delay_ring is null or its struct_size does not match%s");
+    RolloutDelayParams rp;
+    if (pool) {
+        if (int rc = rollout_pool_params(h, r, pool, bot_member, bot_member != -1, rp)) return rc;
+    } else {
+        if (int rc = rollout_mlp_params(h, r, rp)) return rc;
+        if (bot_member != -1) return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_delayed: bot_member must be -1 without a pool%s");
+        rp.pool = {};
+        rp.bot_member = -1;
+    }
+    if (ring->depth < 2 || ring->pos < 0 || ring->pos >= ring->depth)
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_delay_ring: depth must be frame_delay + 1 >= 2 and 0 <= pos < depth%s");
+    if (!ring->ring_obs || !ring->ring_frame || !ring->ring_misc || !ring->out_obs || !ring->out_frame || !ring->out_misc)
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_delay_ring: null buffer%s");
+    if (((uintptr_t)ring->ring_obs & 15u) || ((uintptr_t)ring->out_obs & 15u) || ((uintptr_t)ring->ring_misc & 3u) ||
+        ((uintptr_t)ring->out_misc & 3u))
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_delay_ring: obs buffers must be 16-byte, misc buffers 4-byte aligned%s");
+    rp.ring = { (float4 *)ring->ring_obs, ring->ring_frame, (uint32_t *)ring->ring_misc, (float4 *)ring->out_obs, ring->out_frame,
+                (uint32_t *)ring->out_misc, ring->depth, ring->pos };
+    CUDA_TRY(cudaSetDevice(h->cfg.device));
+    CUDA_TRY(launch_rollout_delayed(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
+    h->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return FG_OK;
 }
 
 int64_t fg_launch_count(fg_handle *h) { return h ? h->launches : 0; }

@@ -25,10 +25,16 @@
 // into the horizon loop of the P2POL = false kernel: RNG plane loaded and stored, bot queried by reset_env / simulate_frame,
 // no P2 weights and no P2 policy pass; actions_p2 receives the bot's held input at the start of each step, logp_p2 zero.
 // Its battles equal a p2_bot = 1 rollout of the same state (tests/test_opponent_pool_bot.py).
+// Delayed observations (fg_rollout_mlp_delayed, DELAY = true, any of the P2 modes above): every step pushes the battle's
+// new state into the caller's frame_delay ring (delay_ring.cuh, the rule fg_delay_ring_step applies) and the emitted,
+// delayed observation is what both policies read next and what obs[t + 1] receives; the bot, rewards, dones and fused
+// frame skipping see the true state.  Equal to the per-step path with fg_delay_ring_step (tests/test_rollout_frame_delay.py);
+// the DELAY = false instantiations are the kernels as they were.
 // Compiled with -fmad=false like the step kernel; the policy arithmetic uses explicit fmaf.
 #include <stdlib.h>
 #include <type_traits>
 
+#include "delay_ring.cuh"
 #include "rollout_kernel.h"
 #include "policy_mma.cuh"
 
@@ -49,9 +55,10 @@ struct RolloutSmem {
 };
 
 // ---- opponent pool (fg_rollout_mlp_pool): a CTA's P2 weights are those of the member whose range holds its battles ----
-template <bool POOL, bool BOTM> struct RolloutArgs { using type = RolloutParams; };
-template <> struct RolloutArgs<true, false> { using type = RolloutPoolParams; };
-template <> struct RolloutArgs<true, true> { using type = RolloutPoolBotParams; };   // BOTM: one member is the in-game bot
+template <bool POOL, bool BOTM, bool DELAY> struct RolloutArgs { using type = RolloutParams; };
+template <> struct RolloutArgs<true, false, false> { using type = RolloutPoolParams; };
+template <> struct RolloutArgs<true, true, false> { using type = RolloutPoolBotParams; };   // BOTM: one member is the in-game bot
+template <bool POOL, bool BOTM> struct RolloutArgs<POOL, BOTM, true> { using type = RolloutDelayParams; };   // every P2 mode
 
 // member of the CTA whose first battle is `first`: the number of boundaries end[0 .. count - 2] at or below it (end is
 // non-decreasing and first < n = end[count - 1]).  Unrolled with constant indices so that the parameter arrays are read
@@ -75,10 +82,63 @@ __device__ __forceinline__ void pool_flush(const RolloutPool &pool, int m, const
     if (pool.stats && tid < 4 && s_stats[tid]) atomicAdd(&pool.stats[(size_t)m * 4 + tid], s_stats[tid]);
 }
 
+// ---- frame_delay queue (fg_rollout_mlp_delayed, DELAY = true): one lane's queue state across the horizon ----
+// Step t pushes the battle's new state at ring position (pos + t) % depth exactly as fg_delay_ring_step does after an
+// fg_step (delay_ring_push); the emitted, delayed observation replaces the true one in obs[t + 1] and in the policy's input
+// rows.  The entry to emit and the newest entry's frame are loaded before the frame update (prefetch): the same thread
+// wrote them in an earlier step, and their latency hides under the frame update instead of lengthening the chain from
+// policy to frame update.  The DELAY = false version is empty and its calls compile to nothing.
+template <bool DELAY> struct DelayQueue {
+    template <class RP> __device__ __forceinline__ DelayQueue(const RP &, bool, int) {}
+    template <class RP> __device__ __forceinline__ void prefetch(const RP &, bool, int) {}
+    template <class RP> __device__ __forceinline__ void push(const RP &, int, int32_t, uint32_t, const float4 *, float4 &, float4 &) {}
+    template <class RP> __device__ __forceinline__ void finish(const RP &, int, float4, float4) const {}
+    template <class RP> __device__ __forceinline__ void advance(const RP &) {}
+};
+template <> struct DelayQueue<true> {
+    int slot;                   // (pos + t) % depth
+    int32_t shown_frame;        // info frame and misc of the delayed state emitted last (what out_* receive at the end)
+    uint32_t shown_misc;
+    DelayEntry oldest;          // slot + 1: the entry this step emits
+    int32_t newest_frame;       // frame of slot - 1
+
+    template <class RP> static __device__ __forceinline__ DelayRingRef ref(const RP &rp) {
+        return { rp.ring.obs, rp.ring.frame, rp.ring.misc, (size_t)rp.sim.n };
+    }
+    template <class RP> __device__ __forceinline__ DelayQueue(const RP &rp, bool valid, int i) : slot(rp.ring.pos) {
+        shown_frame = valid ? rp.ring.out_frame[i] : 0;
+        shown_misc = valid ? rp.ring.out_misc[i] : 0u;
+    }
+    template <class RP> __device__ __forceinline__ void prefetch(const RP &rp, bool valid, int i) {
+        if (valid) {
+            const int d = rp.ring.depth;
+            oldest = ref(rp).load(slot + 1 == d ? 0 : slot + 1, i);
+            newest_frame = rp.ring.frame[(size_t)(slot == 0 ? d - 1 : slot - 1) * rp.sim.n + i];
+        }
+    }
+    // a, b: the step's observation in, the delayed one out; shown_obs: the lane's policy input row (the last emitted
+    // observation, which a battle that did not advance keeps)
+    template <class RP>
+    __device__ __forceinline__ void push(const RP &rp, int i, int32_t frame, uint32_t misc, const float4 *shown_obs, float4 &a, float4 &b) {
+        const DelayEntry now = { a, b, frame, misc };
+        DelayEntry emit;
+        if (delay_ring_push(ref(rp), i, rp.ring.depth, slot, false, now, oldest, newest_frame, emit)) {
+            a = emit.a; b = emit.b; shown_frame = emit.frame; shown_misc = emit.misc;
+        } else {
+            a = shown_obs[0]; b = shown_obs[1];
+        }
+    }
+    template <class RP> __device__ __forceinline__ void finish(const RP &rp, int i, float4 a, float4 b) const {
+        rp.ring.out_obs[2 * (size_t)i] = a; rp.ring.out_obs[2 * (size_t)i + 1] = b;
+        rp.ring.out_frame[i] = shown_frame; rp.ring.out_misc[i] = shown_misc;
+    }
+    template <class RP> __device__ __forceinline__ void advance(const RP &rp) { slot = slot + 1 == rp.ring.depth ? 0 : slot + 1; }
+};
+
 // One CTA's whole horizon.  BOT (opponent pool with the in-game bot as a member, the CTA in the bot's range): P2 is the
 // bot exactly as in the P2POL = false kernel, in the P2POL shared-memory layout, with no P2 weights staged or policy pass.
 // (tid is read in the kernel itself, where the compiler bounds it by __launch_bounds__.)
-template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL, bool BOT, class RP>
+template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL, bool BOT, bool DELAY, class RP>
 __device__ __forceinline__ void rollout_cta(const RP &rp, const int tid) {
     using SM = RolloutSmem<H, E, W, P2POL>;
     using PL = typename SM::PL;
@@ -130,6 +190,7 @@ __device__ __forceinline__ void rollout_cta(const RP &rp, const int tid) {
     StatAcc acc = { 0u, 0u, 0u, 0u };
     uint32_t frames_since_flush = 0u;
     const int K = p.frame_skip;
+    DelayQueue<DELAY> dq(rp, valid, i);
 
     for (int t = 0; t < horizon; t++) {
         // ---- policy phase (two CTA barriers inside) ----
@@ -181,6 +242,7 @@ __device__ __forceinline__ void rollout_cta(const RP &rp, const int tid) {
         if (sim_thread) {
             double reward = 0.0;
             bool terminal = false, ran = false;
+            if constexpr (DELAY) dq.prefetch(rp, valid, i);
             if (valid) {
                 if ((e.misc >> FGM_DONE_SHIFT) & 1u) {                  // next-step autoreset: this step only resets
                     reset_env<false, kP2Bot>(T, e, p.stale_intro != 0);
@@ -217,14 +279,16 @@ __device__ __forceinline__ void rollout_cta(const RP &rp, const int tid) {
             if (valid) {
                 StepOutputs o;
                 make_outputs(e, o);
-                const float4 a = make_float4(o.obs[0], o.obs[1], o.obs[2], o.obs[3]), b = make_float4(o.obs[4], o.obs[5], o.obs[6], o.obs[7]);
+                float4 a = make_float4(o.obs[0], o.obs[1], o.obs[2], o.obs[3]), b = make_float4(o.obs[4], o.obs[5], o.obs[6], o.obs[7]);
+                if constexpr (DELAY) dq.push(rp, i, e.frame, o.info_misc, obs_s + 2 * stid, a, b);       // DELAY: a, b become the delayed observation
                 const size_t dst = ((size_t)(t + 1) * n + i) * 2;
                 rp.obs[dst] = a; rp.obs[dst + 1] = b;
                 rp.rewards[(size_t)t * n + i] = (float)reward;
                 rp.dones[(size_t)t * n + i] = terminal ? 1 : 0;
                 obs_s[2 * stid] = a; obs_s[2 * stid + 1] = b;
-                if (t == horizon - 1) { p.info_frame[i] = e.frame; p.info_misc[i] = o.info_misc; }
+                if (t == horizon - 1) { p.info_frame[i] = e.frame; p.info_misc[i] = o.info_misc; if constexpr (DELAY) dq.finish(rp, i, a, b); }
             }
+            if constexpr (DELAY) dq.advance(rp);
             frames_since_flush += (uint32_t)K;                          // uniform across the warp
             if (frames_since_flush >= kStatFlushFrames) { flush_stats(acc, s_stats, lane); frames_since_flush = 0u; }
         }
@@ -239,16 +303,16 @@ __device__ __forceinline__ void rollout_cta(const RP &rp, const int tid) {
     if constexpr (POOL) pool_flush(rp.pool, member, s_stats, tid);
 }
 
-template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL = false, bool BOTM = false>
-__global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutArgs<POOL, BOTM>::type rp) {
+template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL = false, bool BOTM = false, bool DELAY = false>
+__global__ void __launch_bounds__(32 * W) rollout_kernel(const typename RolloutArgs<POOL, BOTM, DELAY>::type rp) {
     const int tid = threadIdx.x;
     if constexpr (BOTM) {                                       // CTA-uniform: a CTA's battles belong to one member
         if (pool_member(rp.pool, (long long)blockIdx.x * RolloutSmem<H, E, W, P2POL>::kEnvs) == rp.bot_member) {
-            rollout_cta<H, E, W, DENSE, P2POL, SKIP, POOL, true>(rp, tid);
+            rollout_cta<H, E, W, DENSE, P2POL, SKIP, POOL, true, DELAY>(rp, tid);
             return;
         }
     }
-    rollout_cta<H, E, W, DENSE, P2POL, SKIP, POOL, false>(rp, tid);
+    rollout_cta<H, E, W, DENSE, P2POL, SKIP, POOL, false, DELAY>(rp, tid);
 }
 
 // ---- tensor-core version (H <= 64): every WARP owns 16 MT battles for the whole horizon -- policy (policy_mma.cuh: mma.sync
@@ -275,7 +339,7 @@ struct RolloutMmaSmem {
 #define FG_ROLLOUT_MT2_MIN_BLOCKS 1
 #endif
 // One CTA's whole horizon; BOT as in rollout_cta.
-template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL, bool BOT, class RP>
+template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL, bool BOT, bool DELAY, class RP>
 __device__ __forceinline__ void rollout_mma_cta(const RP &rp, const int tid) {
     using SM = RolloutMmaSmem<H, W, P2POL>;
     constexpr bool kP2Pol = P2POL && !BOT;
@@ -322,6 +386,7 @@ __device__ __forceinline__ void rollout_mma_cta(const RP &rp, const int tid) {
     StatAcc acc = { 0u, 0u, 0u, 0u };
     uint32_t frames_since_flush = 0u;
     const int K = p.frame_skip;
+    DelayQueue<DELAY> dq(rp, valid, i);
 
     for (int t = 0; t < horizon; t++) {
         // ---- policy: the warp's battles through the MLP on the tensor cores, then one lane per battle samples ----
@@ -360,6 +425,7 @@ __device__ __forceinline__ void rollout_mma_cta(const RP &rp, const int tid) {
         // ---- FootsiesEnv.step for the warp's battles (same order of events as step_kernel) ----
         double reward = 0.0;
         bool terminal = false, ran = false;
+        if constexpr (DELAY) dq.prefetch(rp, valid, i);
         if (valid) {
             if ((e.misc >> FGM_DONE_SHIFT) & 1u) {                      // next-step autoreset: this step only resets
                 reset_env<false, kP2Bot>(T, e, p.stale_intro != 0);
@@ -394,14 +460,16 @@ __device__ __forceinline__ void rollout_mma_cta(const RP &rp, const int tid) {
         if (valid) {
             StepOutputs o;
             make_outputs(e, o);
-            const float4 a = make_float4(o.obs[0], o.obs[1], o.obs[2], o.obs[3]), b = make_float4(o.obs[4], o.obs[5], o.obs[6], o.obs[7]);
+            float4 a = make_float4(o.obs[0], o.obs[1], o.obs[2], o.obs[3]), b = make_float4(o.obs[4], o.obs[5], o.obs[6], o.obs[7]);
+            if constexpr (DELAY) dq.push(rp, i, e.frame, o.info_misc, reinterpret_cast<const float4 *>(obs_w) + 2 * lane, a, b);   // DELAY: delayed a, b
             const size_t dst = ((size_t)(t + 1) * n + i) * 2;
             rp.obs[dst] = a; rp.obs[dst + 1] = b;
             rp.rewards[(size_t)t * n + i] = (float)reward;
             rp.dones[(size_t)t * n + i] = terminal ? 1 : 0;
             reinterpret_cast<float4 *>(obs_w)[2 * lane] = a; reinterpret_cast<float4 *>(obs_w)[2 * lane + 1] = b;
-            if (t == horizon - 1) { p.info_frame[i] = e.frame; p.info_misc[i] = o.info_misc; }
+            if (t == horizon - 1) { p.info_frame[i] = e.frame; p.info_misc[i] = o.info_misc; if constexpr (DELAY) dq.finish(rp, i, a, b); }
         }
+        if constexpr (DELAY) dq.advance(rp);
         frames_since_flush += (uint32_t)K;                              // uniform across the warp
         if (frames_since_flush >= kStatFlushFrames) { flush_stats(acc, s_stats, lane); frames_since_flush = 0u; }
         __syncwarp();                                                   // observation rows are in place for the next policy pass
@@ -413,41 +481,40 @@ __device__ __forceinline__ void rollout_mma_cta(const RP &rp, const int tid) {
     if constexpr (POOL) pool_flush(rp.pool, member, s_stats, tid);
 }
 
-template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL = false, bool BOTM = false>
+template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL = false, bool BOTM = false, bool DELAY = false>
 __global__ void __launch_bounds__(32 * W, (MT == 2 && !P2POL) ? FG_ROLLOUT_MT2_MIN_BLOCKS : 1)
-rollout_mma_kernel(const typename RolloutArgs<POOL, BOTM>::type rp) {
+rollout_mma_kernel(const typename RolloutArgs<POOL, BOTM, DELAY>::type rp) {
     const int tid = threadIdx.x;
     if constexpr (BOTM) {                                           // CTA-uniform: a CTA's battles belong to one member
         if (pool_member(rp.pool, (long long)blockIdx.x * (16 * MT * W)) == rp.bot_member) {
-            rollout_mma_cta<H, W, MT, DENSE, P2POL, SKIP, POOL, true>(rp, tid);
+            rollout_mma_cta<H, W, MT, DENSE, P2POL, SKIP, POOL, true, DELAY>(rp, tid);
             return;
         }
     }
-    rollout_mma_cta<H, W, MT, DENSE, P2POL, SKIP, POOL, false>(rp, tid);
+    rollout_mma_cta<H, W, MT, DENSE, P2POL, SKIP, POOL, false, DELAY>(rp, tid);
 }
 
 // RP = RolloutParams, or RolloutPoolParams for the opponent-pool instantiations (POOL), or RolloutPoolBotParams for those
-// with the in-game bot as a member (POOL and BOTM)
+// with the in-game bot as a member (POOL and BOTM); the frame_delay kernels (RolloutDelayParams) are dispatched below
 template <class RP> constexpr bool kIsPoolBot = std::is_same<RP, RolloutPoolBotParams>::value;
 template <class RP> constexpr bool kIsPool = std::is_same<RP, RolloutPoolParams>::value || kIsPoolBot<RP>;
 
-template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, class RP>
+template <int H, int W, int MT, bool DENSE, bool P2POL, bool SKIP, bool POOL, bool BOTM, bool DELAY, class RP>
 static cudaError_t launch_rollout_mma_s(cudaStream_t s, const RP &rp) {
-    constexpr bool POOL = kIsPool<RP>, BOTM = kIsPoolBot<RP>;
     constexpr size_t bytes = RolloutMmaSmem<H, W, P2POL>::kBytes;
     static fg::DeviceOnceFlags configured;
     if (cudaError_t e = fg::configure_once_per_device(configured, [] {
-            return cudaFuncSetAttribute(rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL, BOTM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
+            return cudaFuncSetAttribute(rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL, BOTM, DELAY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
         return e;
     constexpr int kEnvs = 16 * MT * W;
     const int grid = (rp.sim.n + kEnvs - 1) / kEnvs;
-    rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL, BOTM><<<grid, 32 * W, bytes, s>>>(rp);
+    rollout_mma_kernel<H, W, MT, DENSE, P2POL, SKIP, POOL, BOTM, DELAY><<<grid, 32 * W, bytes, s>>>(rp);
     return cudaSuccess;
 }
 template <int H, int W, bool DENSE, class RP>
 static cudaError_t launch_rollout_mma_w(int mt, cudaStream_t s, const RP &rp) {
     const bool skip = rp.sim.skip_unactionable != 0;
-#define FG_MMA_GO(MT, P2, SK) launch_rollout_mma_s<H, W, MT, DENSE, P2, SK>(s, rp)
+#define FG_MMA_GO(MT, P2, SK) launch_rollout_mma_s<H, W, MT, DENSE, P2, SK, kIsPool<RP>, kIsPoolBot<RP>, false>(s, rp)
     if (kIsPool<RP> || rp.p2_policy) {
         if (mt == 1) return skip ? FG_MMA_GO(1, true, true) : FG_MMA_GO(1, true, false);
         return skip ? FG_MMA_GO(2, true, true) : FG_MMA_GO(2, true, false);
@@ -459,13 +526,12 @@ static cudaError_t launch_rollout_mma_w(int mt, cudaStream_t s, const RP &rp) {
 #undef FG_MMA_GO
     return cudaErrorInvalidValue;
 }
-template <int H, bool DENSE, class RP>
-static cudaError_t launch_rollout_mma(cudaStream_t s, const RP &rp) {
+inline int rollout_mt(int n) {
     // Measured (profiles/r02f_rollout_mma.log, H = 64, us per step, 16-battle / 32-battle warps / round-1 FFMA2 kernel):
     // 16 384 battles 4.49 / 5.90 / 6.37; 131 072: 28.0 / 31.3 / -; 1 Mi: 216 / 227 / 262 -- more, lighter warps hide the
     // simulator's latency under the neighbours' tensor-core phases at every size, so 16-battle warps are the default
     // (developer knob: FOOTSIES_B200_ROLLOUT_MT = 1 | 2).
-    int mt = rp.sim.n >= 131072 ? 2 : 1;
+    int mt = n >= 131072 ? 2 : 1;
     if (const char *v = getenv("FOOTSIES_B200_ROLLOUT_MT")) mt = atoi(v) == 2 ? 2 : 1;
     // (7-warp CTAs, which would spread 16 384 battles evenly as 147 x 112, measured 4.55 us per step against 4.46 for 4 warps.)
     // (8-battle warps -- half-empty M tiles, twice the warps, 124 registers -- are the same bits and SLOWER from 8192 battles up:
@@ -474,25 +540,30 @@ static cudaError_t launch_rollout_mma(cudaStream_t s, const RP &rp) {
     // profiles/r03h_rollout_half_tiles.log, r03i_rollout_stagger.log.  Step time against batch size -- 4096: 2.46, 8192: 2.48,
     // 16 384: 3.35, 32 768: 6.33 -- says the kernel leaves the latency-bound regime right at one CTA per SM.)
     // Two policies (self-play): 32-battle warps from 131 072 battles up (1 Mi: 479 us per step against 567).
-    return launch_rollout_mma_w<H, 4, DENSE>(mt, s, rp);
+    return mt;
+}
+template <int H, bool DENSE, class RP>
+static cudaError_t launch_rollout_mma(cudaStream_t s, const RP &rp) {
+    return launch_rollout_mma_w<H, 4, DENSE>(rollout_mt(rp.sim.n), s, rp);
 }
 
-template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, class RP>
+template <int H, int E, int W, bool DENSE, bool P2POL, bool SKIP, bool POOL, bool BOTM, bool DELAY, class RP>
 static cudaError_t launch_rollout_s(cudaStream_t s, const RP &rp) {
-    constexpr bool POOL = kIsPool<RP>, BOTM = kIsPoolBot<RP>;
     constexpr size_t bytes = RolloutSmem<H, E, W, P2POL>::kBytes;
     static fg::DeviceOnceFlags configured;
     if (cudaError_t e = fg::configure_once_per_device(configured, [] {
-            return cudaFuncSetAttribute(rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL, BOTM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
+            return cudaFuncSetAttribute(rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL, BOTM, DELAY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes); }))
         return e;
     constexpr int kEnvs = RolloutSmem<H, E, W, P2POL>::kEnvs;
     const int grid = (rp.sim.n + kEnvs - 1) / kEnvs;
-    rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL, BOTM><<<grid, 32 * W, bytes, s>>>(rp);
+    rollout_kernel<H, E, W, DENSE, P2POL, SKIP, POOL, BOTM, DELAY><<<grid, 32 * W, bytes, s>>>(rp);
     return cudaSuccess;
 }
 template <int H, int E, int W, bool DENSE, bool P2POL, class RP>
 static cudaError_t launch_rollout_v(cudaStream_t s, const RP &rp) {
-    return rp.sim.skip_unactionable ? launch_rollout_s<H, E, W, DENSE, P2POL, true>(s, rp) : launch_rollout_s<H, E, W, DENSE, P2POL, false>(s, rp);
+    constexpr bool POOL = kIsPool<RP>, BOTM = kIsPoolBot<RP>;
+    return rp.sim.skip_unactionable ? launch_rollout_s<H, E, W, DENSE, P2POL, true, POOL, BOTM, false>(s, rp)
+                                    : launch_rollout_s<H, E, W, DENSE, P2POL, false, POOL, BOTM, false>(s, rp);
 }
 
 template <int H, bool DENSE, class RP>
@@ -514,8 +585,35 @@ static cudaError_t launch_rollout_h(cudaStream_t s, const RP &rp) {
     return cudaErrorInvalidValue;
 }
 
+// frame_delay rollouts (RolloutDelayParams): instantiated for the shapes launch_rollout_h picks by default only -- the
+// tensor-core kernel with 16- or 32-battle warps for H <= 64 (FOOTSIES_B200_ROLLOUT_MT applies), the FFMA kernel with 2
+// battles per lane for H = 128 -- in every P2 mode.  With a ring bound the developer knobs FOOTSIES_B200_ROLLOUT_FFMA and
+// FOOTSIES_B200_ROLLOUT_E are ignored: the kernels they select have no frame_delay instantiations.
+template <int H, bool DENSE, bool SKIP, bool P2POL, bool POOL, bool BOTM>
+static cudaError_t launch_rollout_delayed_k(cudaStream_t s, const RolloutDelayParams &rp) {
+    if constexpr (H <= kMmaMaxHidden) {
+        return rollout_mt(rp.sim.n) == 1 ? launch_rollout_mma_s<H, 4, 1, DENSE, P2POL, SKIP, POOL, BOTM, true>(s, rp)
+                                         : launch_rollout_mma_s<H, 4, 2, DENSE, P2POL, SKIP, POOL, BOTM, true>(s, rp);
+    } else {
+        return launch_rollout_s<H, 2, kPolicyWarps, DENSE, P2POL, SKIP, POOL, BOTM, true>(s, rp);
+    }
+}
+template <int H, bool DENSE, bool SKIP>
+static cudaError_t launch_rollout_delayed_p(cudaStream_t s, const RolloutDelayParams &rp) {
+    if (rp.pool.count > 0)
+        return rp.bot_member >= 0 ? launch_rollout_delayed_k<H, DENSE, SKIP, true, true, true>(s, rp)
+                                  : launch_rollout_delayed_k<H, DENSE, SKIP, true, true, false>(s, rp);
+    return rp.p2_policy ? launch_rollout_delayed_k<H, DENSE, SKIP, true, false, false>(s, rp)
+                        : launch_rollout_delayed_k<H, DENSE, SKIP, false, false, false>(s, rp);
+}
+template <int H, bool DENSE>
+static cudaError_t launch_rollout_delayed_h(cudaStream_t s, const RolloutDelayParams &rp) {
+    return rp.sim.skip_unactionable ? launch_rollout_delayed_p<H, DENSE, true>(s, rp) : launch_rollout_delayed_p<H, DENSE, false>(s, rp);
+}
+
 // One translation unit per hidden size and reward mode (build.py compiles this file with -DFG_ROLLOUT_H=.. -DFG_ROLLOUT_DENSE=..
-// so that the kernels compile in parallel) plus one without the defines that holds the dispatcher.
+// so that the kernels compile in parallel; with -DFG_ROLLOUT_DELAY=1 it holds the frame_delay kernels of that pair instead)
+// plus one without the defines that holds the dispatcher.
 #define FG_ROLLOUT_DECL(H, D) cudaError_t launch_rollout_##H##_##D(cudaStream_t s, const RolloutParams &rp)
 FG_ROLLOUT_DECL(32, 0); FG_ROLLOUT_DECL(32, 1); FG_ROLLOUT_DECL(64, 0); FG_ROLLOUT_DECL(64, 1); FG_ROLLOUT_DECL(128, 0); FG_ROLLOUT_DECL(128, 1);
 #define FG_ROLLOUT_POOL_DECL(H, D) cudaError_t launch_rollout_pool_##H##_##D(cudaStream_t s, const RolloutPoolParams &rp)
@@ -524,7 +622,14 @@ FG_ROLLOUT_POOL_DECL(128, 0); FG_ROLLOUT_POOL_DECL(128, 1);
 #define FG_ROLLOUT_POOL_BOT_DECL(H, D) cudaError_t launch_rollout_pool_bot_##H##_##D(cudaStream_t s, const RolloutPoolBotParams &rp)
 FG_ROLLOUT_POOL_BOT_DECL(32, 0); FG_ROLLOUT_POOL_BOT_DECL(32, 1); FG_ROLLOUT_POOL_BOT_DECL(64, 0); FG_ROLLOUT_POOL_BOT_DECL(64, 1);
 FG_ROLLOUT_POOL_BOT_DECL(128, 0); FG_ROLLOUT_POOL_BOT_DECL(128, 1);
-#ifdef FG_ROLLOUT_H
+#define FG_ROLLOUT_DELAY_DECL(H, D) cudaError_t launch_rollout_delayed_##H##_##D(cudaStream_t s, const RolloutDelayParams &rp)
+FG_ROLLOUT_DELAY_DECL(32, 0); FG_ROLLOUT_DELAY_DECL(32, 1); FG_ROLLOUT_DELAY_DECL(64, 0); FG_ROLLOUT_DELAY_DECL(64, 1);
+FG_ROLLOUT_DELAY_DECL(128, 0); FG_ROLLOUT_DELAY_DECL(128, 1);
+#if defined(FG_ROLLOUT_H) && defined(FG_ROLLOUT_DELAY)
+#define FG_ROLLOUT_DEF2(H, D) FG_ROLLOUT_DELAY_DECL(H, D) { return launch_rollout_delayed_h<H, (D != 0)>(s, rp); }
+#define FG_ROLLOUT_DEF(H, D) FG_ROLLOUT_DEF2(H, D)
+FG_ROLLOUT_DEF(FG_ROLLOUT_H, FG_ROLLOUT_DENSE)
+#elif defined(FG_ROLLOUT_H)
 #define FG_ROLLOUT_DEF2(H, D) FG_ROLLOUT_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); } \
     FG_ROLLOUT_POOL_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); } \
     FG_ROLLOUT_POOL_BOT_DECL(H, D) { return launch_rollout_h<H, (D != 0)>(s, rp); }
@@ -552,6 +657,14 @@ cudaError_t launch_rollout_pool_bot(bool dense, cudaStream_t s, const RolloutPoo
     case 32: return dense ? launch_rollout_pool_bot_32_1(s, rp) : launch_rollout_pool_bot_32_0(s, rp);
     case 64: return dense ? launch_rollout_pool_bot_64_1(s, rp) : launch_rollout_pool_bot_64_0(s, rp);
     case 128: return dense ? launch_rollout_pool_bot_128_1(s, rp) : launch_rollout_pool_bot_128_0(s, rp);
+    default: return cudaErrorInvalidValue;
+    }
+}
+cudaError_t launch_rollout_delayed(bool dense, cudaStream_t s, const RolloutDelayParams &rp) {
+    switch (rp.hidden) {
+    case 32: return dense ? launch_rollout_delayed_32_1(s, rp) : launch_rollout_delayed_32_0(s, rp);
+    case 64: return dense ? launch_rollout_delayed_64_1(s, rp) : launch_rollout_delayed_64_0(s, rp);
+    case 128: return dense ? launch_rollout_delayed_128_1(s, rp) : launch_rollout_delayed_128_0(s, rp);
     default: return cudaErrorInvalidValue;
     }
 }

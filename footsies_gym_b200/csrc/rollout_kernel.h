@@ -45,9 +45,27 @@ struct RolloutPoolBotParams : RolloutPoolParams {
     int bot_member;
 };
 
+// Observations delayed by frame_delay = depth - 1 steps (fg_rollout_mlp_delayed): the queue of every battle is the caller's
+// ring (delay_ring.cuh), advanced once per step at position (pos + t) % depth; out_* receive the delayed state after the
+// last step.  One parameter struct for every P2 mode: pool.count = 0 is no pool, bot_member = -1 no bot member.
+struct RolloutRing {
+    float4 *obs;                // [depth][n][2]
+    int32_t *frame;             // [depth][n]
+    uint32_t *misc;             // [depth][n]
+    float4 *out_obs;            // [n][2]
+    int32_t *out_frame;         // [n]
+    uint32_t *out_misc;         // [n]
+    int depth, pos;
+};
+struct RolloutDelayParams : RolloutPoolBotParams {
+    RolloutRing ring;
+};
+
 // P1 = the MLP policy, P2 = the in-game BattleAI or a second MLP policy (p2_policy), autoreset on.  Returns
 // cudaErrorInvalidValue for other hidden sizes.
 cudaError_t launch_rollout(bool dense, cudaStream_t s, const RolloutParams &rp);
+// Any of the modes below or above with the frame_delay queue (P2 from rp.pool when rp.pool.count > 0).
+cudaError_t launch_rollout_delayed(bool dense, cudaStream_t s, const RolloutDelayParams &rp);
 // The same with P2 from an opponent pool (rp.p2_policy = 1; w_p2 is not read).
 cudaError_t launch_rollout_pool(bool dense, cudaStream_t s, const RolloutPoolParams &rp);
 // The same with member rp.bot_member played by the in-game bot (its weights are not read).

@@ -17,6 +17,13 @@ Three policy paths:
     own range of battles, with results per member) runs on this path only (fg_rollout_mlp_pool); one member may be the
     in-game bot, "bot" (fg_rollout_mlp_pool_bot).
 
+An env with frame_delay > 0 runs on every path: the policies act on the delayed observation, as the reference's agent and
+its `opponent(obs, info)` callable do (footsies.py:129-131, 533-535), and obs[t + 1] of the rollout buffer receives the
+delayed observation; rewards and dones are not delayed.  The whole-horizon kernel advances the env's queue inside its one
+launch (fg_rollout_mlp_delayed); the per-step paths run env.step_bound() (which advances the queue with
+fg_delay_ring_step) and copy the delayed observation into the buffer, without a CUDA graph: the ring position is a host
+integer that a captured launch would replay frozen.
+
 With a value network (`value=`), collect() also returns what a PPO update consumes besides the rollout itself: the values
 of all horizon + 1 observation rows (one fg_value_mlp launch for an `MLPValue` with hidden 32 / 64, else one call of the
 torch callable) and GAE advantages / returns (one fg_gae launch), after the rollout on the same stream.
@@ -241,7 +248,11 @@ class RolloutCollector:
     battles actions_p2 holds the bot's input at the start of each step and logp_p2 is 0 (not a log-probability).  A battle
     moved into the bot's range continues its episode with empty bot queues and P2's last held input; the first round
     after env.reset() of a battle in the bot's range starts like such an entry (a self-play env's reset does not ask the
-    bot for its Fight-transition input), every later round exactly as on a bot env."""
+    bot for its Fight-transition input), every later round exactly as on a bot env.
+
+    frame_delay > 0: every policy acts on the delayed observation the env shows (see the module docstring), and obs[0] of
+    each collect() is what the env shows when it starts, so env.step() / env.reset() calls between collects are picked
+    up.  The per-step paths ("step", "torch") run without a CUDA graph then, whatever use_cuda_graph says."""
 
     def __init__(self, env: FootsiesEnv, policy: Callable[[torch.Tensor], torch.Tensor], horizon: int = 128,
                  use_cuda_graph: bool = True, fused=None, seed: int = 0,
@@ -264,8 +275,6 @@ class RolloutCollector:
         kernel (fused=None / True / "horizon"); anything else is a ValueError."""
         if env.by_example:
             raise ValueError("the policy drives P1: create the env with by_example=False")
-        if env.frame_delay:
-            raise ValueError("RolloutCollector binds the env's outputs directly: frame_delay must be 0")
         self.env, self.policy, self.horizon = env, policy, int(horizon)
         self.opponent_policy, self.mirror_opponent = opponent_policy, bool(mirror_opponent)
         if opponent_policy is not None and (env._opponent_mode == "bot" or env.opponent is not None):
@@ -320,7 +329,7 @@ class RolloutCollector:
         self.use_cuda_graph = bool(use_cuda_graph)
         if not env.has_reset:
             env.reset()
-        self.obs[h].copy_(env.obs)                                  # the observation the first step will act on
+        self.obs[h].copy_(env._delayed_obs if env.frame_delay else env.obs)   # what the first step will act on
 
     def _check_pool(self, fused):
         env, pool = self.env, self.opponent_pool
@@ -382,7 +391,8 @@ class RolloutCollector:
 
     def _horizon_launch(self):
         """fg_rollout_mlp (fg_rollout_mlp_pool with an opponent pool, fg_rollout_mlp_pool_bot when the bot is one of its
-        members): the whole horizon in one launch on the current stream."""
+        members, fg_rollout_mlp_delayed for any of them with frame_delay > 0): the whole horizon in one launch on the
+        current stream."""
         env, pol = self.env, self.policy
         l1, l2, l3 = pol.net[0], pol.net[2], pol.net[4]
         r = _capi.FgRolloutBuffers(struct_size=C.sizeof(_capi.FgRolloutBuffers), hidden=pol.hidden, horizon=self.horizon,
@@ -405,7 +415,17 @@ class RolloutCollector:
             if not t.is_contiguous() or t.device != env.device:
                 raise ValueError(f"fused rollout needs contiguous tensors on the env's device ({k})")
             setattr(r, k, t.data_ptr())
-        if self.opponent_pool is not None:
+        if env.frame_delay:
+            depth = env.frame_delay + 1
+            ring = _capi.FgDelayRing(struct_size=C.sizeof(_capi.FgDelayRing), depth=depth, pos=env._ring_pos, reserved0=0)
+            for k, t in dict(ring_obs=env._ring_obs, ring_frame=env._ring_frame, ring_misc=env._ring_misc,
+                             out_obs=env._delayed_obs, out_frame=env._delayed_frame, out_misc=env._delayed_misc).items():
+                setattr(ring, k, t.data_ptr())
+            pool = None if self.opponent_pool is None else C.byref(self._pool_struct())
+            bot = -1 if self._pool_bot is None else self._pool_bot
+            _capi.check(env._lib.fg_rollout_mlp_delayed(env._handle, C.byref(r), pool, bot, C.byref(ring), env._stream()))
+            env._ring_pos = (env._ring_pos + self.horizon) % depth
+        elif self.opponent_pool is not None:
             pool = self._pool_struct()
             if self._pool_bot is None:
                 _capi.check(env._lib.fg_rollout_mlp_pool(env._handle, C.byref(r), C.byref(pool), env._stream()))
@@ -435,6 +455,8 @@ class RolloutCollector:
 
     def _rollout(self):
         env, h = self.env, self.horizon
+        if env.frame_delay:
+            self.obs[h].copy_(env._delayed_obs)                     # what the env shows now (env.step() / reset() since)
         if self.mode == "horizon":
             return self._horizon_launch()
         self.obs[0].copy_(self.obs[h])                              # carry the last observation over
@@ -464,13 +486,16 @@ class RolloutCollector:
                 env.bind_actions(self.actions[t], self.actions_p2[t])
             env.bind_outputs(obs=self.obs[t + 1], reward=self.rewards[t], terminated=self.dones[t])
             env.step_bound()
+            if env.frame_delay:
+                self.obs[t + 1].copy_(env._delayed_obs)             # the queue has taken the true observation already
         self._drawn.add_(h)
 
     def collect(self):
         """Runs one horizon (and with a value network its values and GAE); returns the rollout buffers (views,
         overwritten by the next call)."""
         dev = self.env.device
-        if not self.use_cuda_graph or self.mode == "horizon":      # one launch: nothing for a graph to save
+        # horizon: one launch, nothing for a graph to save; frame_delay: the ring position is a host integer
+        if not self.use_cuda_graph or self.mode == "horizon" or self.env.frame_delay:
             self._one_horizon()
         else:
             if self._graph is None:

@@ -24,7 +24,8 @@ extern "C" {
 
 /* 2 (round 2): fg_env_state.p1_bot_memory, first_env_index argument of fg_policy_mlp_sample[_p2], packed host layout
  * (fg_packed_result, fg_step_host_packed, fg_reset_host_packed, fg_packed_reward_table), fg_host_alloc / fg_host_free.
- * Added since, backward compatible (new entry points only, so still 2): fg_value_mlp, fg_gae, fg_rollout_mlp_pool, fg_rollout_mlp_pool_bot. */
+ * Added since, backward compatible (new entry points only, so still 2): fg_value_mlp, fg_gae, fg_rollout_mlp_pool, fg_rollout_mlp_pool_bot,
+ * fg_rollout_mlp_delayed (with its new fg_delay_ring struct). */
 #define FG_ABI_VERSION 2
 
 typedef enum {
@@ -320,6 +321,29 @@ int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_
  *     exactly the bot handle's round. */
 int32_t fg_rollout_mlp_pool_bot(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool,
                                 int32_t bot_member, void *stream);
+
+/* Whole-horizon rollouts with delayed observations (FootsiesEnv frame_delay, footsies.py:129-131, 502-504, 533-535): any
+ * of the three calls above -- pool = NULL and bot_member = -1 is fg_rollout_mlp; a pool with bot_member = -1 is
+ * fg_rollout_mlp_pool; a pool with bot_member in 0 .. count - 1 is fg_rollout_mlp_pool_bot -- with the frame_delay queue of
+ * every battle advanced inside the launch.  Each call's requirements and checks apply unchanged.
+ *   - Twin contract: bit-identical to `horizon` rounds of { policy sample(s) on the delayed observation; fg_step;
+ *     fg_delay_ring_step(depth, (pos + t) % depth) } on a handle holding the same state.  P1's policy and a policy-driven
+ *     P2 (mirrored or not, a pool member too) read the DELAYED observation, as the reference's `opponent(obs, info)` gets
+ *     the delayed observation; the in-game bot reads the battle state as always.  obs[t + 1] receives the delayed
+ *     observation (what the policy acts on at step t + 1); rewards and dones are not delayed.  Fused frame skipping
+ *     decides on the true state, and the queue advances once per step.
+ *   - The ring is the caller's, in DEVICE memory, laid out as for fg_delay_ring_step; when the call returns it is exactly
+ *     what those `horizon` fg_delay_ring_step calls would leave, and out_* hold the delayed state after the last step (as
+ *     fg_delay_ring_step's out_* do).  The caller advances pos by horizon % depth.
+ *   - obs[0] is still first overwritten with obs[horizon]: keep that row equal to out_obs (the delayed observation the
+ *     env shows) when the battles are stepped or reset between calls. */
+typedef struct {
+    int32_t struct_size, depth, pos, reserved0;   /* depth = frame_delay + 1 >= 2; 0 <= pos < depth              */
+    float *ring_obs; int32_t *ring_frame; uint8_t *ring_misc;   /* as fg_delay_ring_step (16- / 4-byte aligned) */
+    float *out_obs;  int32_t *out_frame;  uint8_t *out_misc;    /* the delayed state after the last step        */
+} fg_delay_ring;
+int32_t fg_rollout_mlp_delayed(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool /* NULL: no pool */,
+                               int32_t bot_member /* -1: none */, const fg_delay_ring *ring, void *stream);
 
 /* Critic side of an actor-critic (PPO) rollout, for any source of rollout buffers.  Handle-free like fg_policy_mlp_sample;
  * errors are reported through fg_policy_last_error().  All pointers are DEVICE pointers.
