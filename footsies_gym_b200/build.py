@@ -79,10 +79,9 @@ def translation_units():
              ("rollout.o", os.path.join(CSRC, "rollout_kernel.cu"), [])]           # the dispatcher
     for hidden in (32, 64, 128):
         for dense in (0, 1):
-            units.append((f"rollout_h{hidden}_d{dense}.o", os.path.join(CSRC, "rollout_kernel.cu"),
-                          [f"-DFG_ROLLOUT_H={hidden}", f"-DFG_ROLLOUT_DENSE={dense}"]))
-            units.append((f"rollout_delay_h{hidden}_d{dense}.o", os.path.join(CSRC, "rollout_kernel.cu"),
-                          [f"-DFG_ROLLOUT_H={hidden}", f"-DFG_ROLLOUT_DENSE={dense}", "-DFG_ROLLOUT_DELAY=1"]))
+            for delay in (0, 1):
+                units.append((f"rollout{'_delay' if delay else ''}_h{hidden}_d{dense}.o", os.path.join(CSRC, "rollout_kernel.cu"),
+                              [f"-DFG_ROLLOUT_H={hidden}", f"-DFG_ROLLOUT_DENSE={dense}", f"-DFG_ROLLOUT_DELAY={delay}"]))
     for kf in (0, 1):
         for b1 in (0, 1):
             for b2 in (0, 1):

@@ -710,38 +710,81 @@ int32_t fg_delay_ring_step(fg_handle *h, int32_t depth, int32_t pos, float *ring
     return FG_OK;
 }
 
-// fg_rollout_mlp's checks and parameter block (also the no-pool case of fg_rollout_mlp_delayed)
-static int32_t rollout_mlp_params(fg_handle *h, const fg_rollout_buffers *r, RolloutParams &rp) {
+// The checks and parameter block every fg_rollout_mlp* entry point shares, in this order: the pool struct (with_pool), the
+// handle, the buffers struct, the handle's configuration, P2 (the pool and its bot member with a pool, the second policy's
+// weights without one), hidden size, horizon, buffer pointers and alignment.  No pool: pool.count = 0, bot_member = -1.
+// ring.depth is left 0 (no frame_delay).
+static int32_t rollout_params(fg_handle *h, const fg_rollout_buffers *r, bool with_pool, const fg_opponent_pool *pool, bool with_bot,
+                              int32_t bot_member, RolloutParams &rp) {
+    if (with_pool && (!pool || pool->struct_size != (int32_t)sizeof(fg_opponent_pool)))
+        return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool is null or its struct_size does not match%s");
     if (int rc = check_bound(h)) return rc;
     if (!r || r->struct_size != (int32_t)sizeof(fg_rollout_buffers))
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers is null or its struct_size does not match%s");
     if (h->cfg.p1_bot || !h->cfg.autoreset || h->buf.step_mask)
-        return fail(FG_ERR_INVALID_STATE, "fg_rollout_mlp needs P1 = policy, autoreset on, no step mask "
-                                          "(use fg_policy_mlp_sample + fg_step for other configurations)%s");
+        return fail(FG_ERR_INVALID_STATE, with_pool ? "fg_rollout_mlp_pool needs P1 = policy, autoreset on, no step mask%s"
+                                                    : "fg_rollout_mlp needs P1 = policy, autoreset on, no step mask "
+                                                      "(use fg_policy_mlp_sample + fg_step for other configurations)%s");
+    const int64_t n = h->cfg.num_envs;
     const bool p2_policy = !h->cfg.p2_bot;
-    if (p2_policy && (!r->p2_scale || !r->p2_w1 || !r->p2_b1 || !r->p2_w2 || !r->p2_b2 || !r->p2_w3 || !r->p2_b3 || !r->actions_p2 ||
-                      !r->logp_p2 || ((uintptr_t)r->p2_w2 & 15u)))
+    if (with_pool) {
+        if (!p2_policy)
+            return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_pool needs p2_bot = 0: the pool plays P2 (the in-game bot cannot be a member)%s");
+        if (pool->count < 1 || pool->count > FG_POOL_MAX) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.count must be in 1..16%s");
+        if (with_bot && (bot_member < 0 || bot_member >= pool->count))
+            return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_pool_bot: bot_member must be in 0 .. fg_opponent_pool.count - 1%s");
+        for (int m = 0; m < pool->count; m++) {
+            const int64_t lo = m ? pool->end[m - 1] : 0, e = pool->end[m];
+            if (e < lo || e > n) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end must be non-decreasing and at most num_envs%s");
+            if (e % FG_POOL_BLOCK && e != n)
+                return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end: every boundary must be a multiple of FG_POOL_BLOCK (128) or num_envs%s");
+            if (with_bot && m == bot_member) continue;              // the bot's weight pointers are not read
+            const fg_mlp_weights &w = pool->member[m];
+            if (!w.scale || !w.w1 || !w.b1 || !w.w2 || !w.b2 || !w.w3 || !w.b3)
+                return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool: null member weight pointer%s");
+            if ((uintptr_t)w.w2 & 15u) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool: member w2 must be 16-byte aligned%s");
+        }
+        if (pool->end[pool->count - 1] != n) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end[count - 1] must be num_envs%s");
+        if ((uintptr_t)pool->stats & 7u) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.stats must be 8-byte aligned%s");
+    } else if (p2_policy && (!r->p2_scale || !r->p2_w1 || !r->p2_b1 || !r->p2_w2 || !r->p2_b2 || !r->p2_w3 || !r->p2_b3 ||
+                             !r->actions_p2 || !r->logp_p2 || ((uintptr_t)r->p2_w2 & 15u))) {
         return fail(FG_ERR_INVALID_ARGUMENT, "p2_bot = 0: fg_rollout_buffers needs the P2 policy (p2_* weights, 16-byte aligned p2_w2, "
                                              "actions_p2, logp_p2)%s");
-    if (r->hidden != 32 && r->hidden != 64 && r->hidden != 128) return fail(FG_ERR_INVALID_ARGUMENT, "hidden size must be 32, 64 or 128%s");
+    }
+    if (r->hidden != 32 && r->hidden != 64 && r->hidden != 128)
+        return fail(FG_ERR_INVALID_ARGUMENT, with_pool ? "hidden size must be 32, 64 or 128 (the learner's and every member's)%s"
+                                                       : "hidden size must be 32, 64 or 128%s");
     if (r->horizon < 1) return fail(FG_ERR_INVALID_ARGUMENT, "horizon must be positive%s");
-    if (!r->scale || !r->w1 || !r->b1 || !r->w2 || !r->b2 || !r->w3 || !r->b3 || !r->obs || !r->actions || !r->logp || !r->rewards || !r->dones)
-        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers: null pointer%s");
+    if (!r->scale || !r->w1 || !r->b1 || !r->w2 || !r->b2 || !r->w3 || !r->b3 || !r->obs || !r->actions || !r->logp || !r->rewards ||
+        !r->dones || (with_pool && (!r->actions_p2 || !r->logp_p2)))
+        return fail(FG_ERR_INVALID_ARGUMENT, with_pool ? "fg_rollout_buffers: null pointer (actions_p2 and logp_p2 are required)%s"
+                                                       : "fg_rollout_buffers: null pointer%s");
     if (((uintptr_t)r->obs & 15u) || ((uintptr_t)r->w2 & 15u)) return fail(FG_ERR_INVALID_ARGUMENT, "obs and w2 must be 16-byte aligned%s");
+    rp = {};
     rp.sim = make_params(h);
     rp.w = { r->scale, r->w1, r->b1, r->w2, r->b2, r->w3, r->b3 };
     rp.seed = r->seed; rp.counter_base = (const unsigned long long *)r->counter_base;
     rp.hidden = r->hidden; rp.horizon = r->horizon;
     rp.obs = (float4 *)r->obs; rp.actions = r->actions; rp.logp = r->logp; rp.rewards = r->rewards; rp.dones = r->dones;
     rp.p2_policy = p2_policy; rp.p2_mirror = p2_policy && r->p2_mirror;
-    rp.w_p2 = { r->p2_scale, r->p2_w1, r->p2_b1, r->p2_w2, r->p2_b2, r->p2_w3, r->p2_b3 };
+    rp.w_p2 = { r->p2_scale, r->p2_w1, r->p2_b1, r->p2_w2, r->p2_b2, r->p2_w3, r->p2_b3 };   // not read with a pool
     rp.seed_p2 = r->p2_seed; rp.actions_p2 = r->actions_p2; rp.logp_p2 = r->logp_p2;
+    if (with_pool) {
+        for (int m = 0; m < FG_POOL_MAX; m++) {
+            const bool used = m < pool->count;
+            const fg_mlp_weights &w = pool->member[used ? m : 0];
+            rp.pool.member[m] = { w.scale, w.w1, w.b1, w.w2, w.b2, w.w3, w.b3 };
+            rp.pool.end[m] = used ? pool->end[m] : n;
+        }
+        rp.pool.count = pool->count;
+        rp.pool.stats = (unsigned long long *)pool->stats;
+    }
+    rp.bot_member = with_bot ? bot_member : -1;
     return FG_OK;
 }
 
-int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) {
-    RolloutParams rp;
-    if (int rc = rollout_mlp_params(h, r, rp)) return rc;
+// the launch every fg_rollout_mlp* entry point ends with, once its checks have passed
+static int32_t rollout_launch(fg_handle *h, const RolloutParams &rp, void *stream) {
     CUDA_TRY(cudaSetDevice(h->cfg.device));
     CUDA_TRY(launch_rollout(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
     h->launches++;
@@ -749,97 +792,32 @@ int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) 
     return FG_OK;
 }
 
-// fg_rollout_mlp_pool's and fg_rollout_mlp_pool_bot's checks and parameter block (bot_member = -1 without the bot)
-static int32_t rollout_pool_params(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
-                                   bool with_bot, RolloutPoolBotParams &rp) {
-    if (!pool || pool->struct_size != (int32_t)sizeof(fg_opponent_pool))
-        return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool is null or its struct_size does not match%s");
-    if (int rc = check_bound(h)) return rc;
-    if (!r || r->struct_size != (int32_t)sizeof(fg_rollout_buffers))
-        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers is null or its struct_size does not match%s");
-    if (h->cfg.p1_bot || !h->cfg.autoreset || h->buf.step_mask)
-        return fail(FG_ERR_INVALID_STATE, "fg_rollout_mlp_pool needs P1 = policy, autoreset on, no step mask%s");
-    if (h->cfg.p2_bot)
-        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_pool needs p2_bot = 0: the pool plays P2 (the in-game bot cannot be a member)%s");
-    if (pool->count < 1 || pool->count > FG_POOL_MAX) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.count must be in 1..16%s");
-    if (with_bot && (bot_member < 0 || bot_member >= pool->count))
-        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_pool_bot: bot_member must be in 0 .. fg_opponent_pool.count - 1%s");
-    const int64_t n = h->cfg.num_envs;
-    for (int m = 0; m < pool->count; m++) {
-        const int64_t lo = m ? pool->end[m - 1] : 0, e = pool->end[m];
-        if (e < lo || e > n) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end must be non-decreasing and at most num_envs%s");
-        if (e % FG_POOL_BLOCK && e != n)
-            return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end: every boundary must be a multiple of FG_POOL_BLOCK (128) or num_envs%s");
-        if (with_bot && m == bot_member) continue;                  // the bot's weight pointers are not read
-        const fg_mlp_weights &w = pool->member[m];
-        if (!w.scale || !w.w1 || !w.b1 || !w.w2 || !w.b2 || !w.w3 || !w.b3)
-            return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool: null member weight pointer%s");
-        if ((uintptr_t)w.w2 & 15u) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool: member w2 must be 16-byte aligned%s");
-    }
-    if (pool->end[pool->count - 1] != n) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.end[count - 1] must be num_envs%s");
-    if ((uintptr_t)pool->stats & 7u) return fail(FG_ERR_INVALID_ARGUMENT, "fg_opponent_pool.stats must be 8-byte aligned%s");
-    if (r->hidden != 32 && r->hidden != 64 && r->hidden != 128)
-        return fail(FG_ERR_INVALID_ARGUMENT, "hidden size must be 32, 64 or 128 (the learner's and every member's)%s");
-    if (r->horizon < 1) return fail(FG_ERR_INVALID_ARGUMENT, "horizon must be positive%s");
-    if (!r->scale || !r->w1 || !r->b1 || !r->w2 || !r->b2 || !r->w3 || !r->b3 || !r->obs || !r->actions || !r->logp || !r->rewards ||
-        !r->dones || !r->actions_p2 || !r->logp_p2)
-        return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_buffers: null pointer (actions_p2 and logp_p2 are required)%s");
-    if (((uintptr_t)r->obs & 15u) || ((uintptr_t)r->w2 & 15u)) return fail(FG_ERR_INVALID_ARGUMENT, "obs and w2 must be 16-byte aligned%s");
-    rp.sim = make_params(h);
-    rp.w = { r->scale, r->w1, r->b1, r->w2, r->b2, r->w3, r->b3 };
-    rp.seed = r->seed; rp.counter_base = (const unsigned long long *)r->counter_base;
-    rp.hidden = r->hidden; rp.horizon = r->horizon;
-    rp.obs = (float4 *)r->obs; rp.actions = r->actions; rp.logp = r->logp; rp.rewards = r->rewards; rp.dones = r->dones;
-    rp.p2_policy = 1; rp.p2_mirror = r->p2_mirror != 0;
-    rp.w_p2 = {};
-    rp.seed_p2 = r->p2_seed; rp.actions_p2 = r->actions_p2; rp.logp_p2 = r->logp_p2;
-    for (int m = 0; m < FG_POOL_MAX; m++) {
-        const bool used = m < pool->count;
-        const fg_mlp_weights &w = pool->member[used ? m : 0];
-        rp.pool.member[m] = { w.scale, w.w1, w.b1, w.w2, w.b2, w.w3, w.b3 };
-        rp.pool.end[m] = used ? pool->end[m] : n;
-    }
-    rp.pool.count = pool->count;
-    rp.pool.stats = (unsigned long long *)pool->stats;
-    rp.bot_member = with_bot ? bot_member : -1;
-    return FG_OK;
-}
-
-// fg_rollout_mlp_pool (bot_member = -1) and fg_rollout_mlp_pool_bot
-static int32_t rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
-                                bool with_bot, void *stream) {
-    RolloutPoolBotParams rp;
-    if (int rc = rollout_pool_params(h, r, pool, bot_member, with_bot, rp)) return rc;
-    CUDA_TRY(cudaSetDevice(h->cfg.device));
-    if (with_bot) CUDA_TRY(launch_rollout_pool_bot(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
-    else CUDA_TRY(launch_rollout_pool(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
-    h->launches++;
-    CUDA_TRY(cudaGetLastError());
-    return FG_OK;
+int32_t fg_rollout_mlp(fg_handle *h, const fg_rollout_buffers *r, void *stream) {
+    RolloutParams rp;
+    if (int rc = rollout_params(h, r, false, nullptr, false, -1, rp)) return rc;
+    return rollout_launch(h, rp, stream);
 }
 
 int32_t fg_rollout_mlp_pool(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, void *stream) {
-    return rollout_mlp_pool(h, r, pool, -1, false, stream);
+    RolloutParams rp;
+    if (int rc = rollout_params(h, r, true, pool, false, -1, rp)) return rc;
+    return rollout_launch(h, rp, stream);
 }
 
 int32_t fg_rollout_mlp_pool_bot(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
                                 void *stream) {
-    return rollout_mlp_pool(h, r, pool, bot_member, true, stream);
+    RolloutParams rp;
+    if (int rc = rollout_params(h, r, true, pool, true, bot_member, rp)) return rc;
+    return rollout_launch(h, rp, stream);
 }
 
 int32_t fg_rollout_mlp_delayed(fg_handle *h, const fg_rollout_buffers *r, const fg_opponent_pool *pool, int32_t bot_member,
                                const fg_delay_ring *ring, void *stream) {
     if (!ring || ring->struct_size != (int32_t)sizeof(fg_delay_ring))
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_delay_ring is null or its struct_size does not match%s");
-    RolloutDelayParams rp;
-    if (pool) {
-        if (int rc = rollout_pool_params(h, r, pool, bot_member, bot_member != -1, rp)) return rc;
-    } else {
-        if (int rc = rollout_mlp_params(h, r, rp)) return rc;
-        if (bot_member != -1) return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_delayed: bot_member must be -1 without a pool%s");
-        rp.pool = {};
-        rp.bot_member = -1;
-    }
+    RolloutParams rp;
+    if (int rc = rollout_params(h, r, pool != nullptr, pool, pool && bot_member != -1, bot_member, rp)) return rc;
+    if (!pool && bot_member != -1) return fail(FG_ERR_INVALID_ARGUMENT, "fg_rollout_mlp_delayed: bot_member must be -1 without a pool%s");
     if (ring->depth < 2 || ring->pos < 0 || ring->pos >= ring->depth)
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_delay_ring: depth must be frame_delay + 1 >= 2 and 0 <= pos < depth%s");
     if (!ring->ring_obs || !ring->ring_frame || !ring->ring_misc || !ring->out_obs || !ring->out_frame || !ring->out_misc)
@@ -849,11 +827,7 @@ int32_t fg_rollout_mlp_delayed(fg_handle *h, const fg_rollout_buffers *r, const 
         return fail(FG_ERR_INVALID_ARGUMENT, "fg_delay_ring: obs buffers must be 16-byte, misc buffers 4-byte aligned%s");
     rp.ring = { (float4 *)ring->ring_obs, ring->ring_frame, (uint32_t *)ring->ring_misc, (float4 *)ring->out_obs, ring->out_frame,
                 (uint32_t *)ring->out_misc, ring->depth, ring->pos };
-    CUDA_TRY(cudaSetDevice(h->cfg.device));
-    CUDA_TRY(launch_rollout_delayed(h->cfg.dense_reward != 0, (cudaStream_t)stream, rp));
-    h->launches++;
-    CUDA_TRY(cudaGetLastError());
-    return FG_OK;
+    return rollout_launch(h, rp, stream);
 }
 
 int64_t fg_launch_count(fg_handle *h) { return h ? h->launches : 0; }

@@ -6,6 +6,28 @@
 
 namespace fgk {
 
+// P2 from an opponent pool: member m plays the battles [end[m - 1], end[m]).  The boundaries are multiples of FG_POOL_BLOCK
+// (or n), so each CTA belongs to one member, stages its weights where the single P2 policy's go and adds its episode
+// results to stats[member][0..3] (optional) when it flushes its statistics at the end.
+struct RolloutPool {
+    fgp::PolicyWeights member[FG_POOL_MAX];
+    long long end[FG_POOL_MAX];
+    int count;
+    unsigned long long *stats;  // [count][4] or null
+};
+
+// Observations delayed by frame_delay = depth - 1 steps: the queue of every battle is the caller's ring (delay_ring.cuh),
+// advanced once per step at position (pos + t) % depth; out_* receive the delayed state after the last step.
+struct RolloutRing {
+    float4 *obs;                // [depth][n][2]
+    int32_t *frame;             // [depth][n]
+    uint32_t *misc;             // [depth][n]
+    float4 *out_obs;            // [n][2]
+    int32_t *out_frame;         // [n]
+    uint32_t *out_misc;         // [n]
+    int depth, pos;
+};
+
 struct RolloutParams {
     Params sim;                 // state planes, statistics, tables, info outputs, n, frame_skip, stale_intro
     fgp::PolicyWeights w;
@@ -24,52 +46,14 @@ struct RolloutParams {
     unsigned long long seed_p2;
     uint8_t *actions_p2;        // [horizon][n]
     float *logp_p2;             // [horizon][n]
+    RolloutPool pool;           // P2 from an opponent pool when pool.count > 0 (then p2_policy = 1 and w_p2 is not read)
+    int bot_member;             // the pool member played by the in-game bot (its weights are not read), or -1
+    RolloutRing ring;           // ring.depth = 0: no frame_delay
 };
 
-// P2 from an opponent pool (fg_rollout_mlp_pool): member m plays the battles [end[m - 1], end[m]).  The boundaries are
-// multiples of FG_POOL_BLOCK (or n), so each CTA belongs to one member, stages its weights where the single P2 policy's go
-// and adds its episode results to stats[member][0..3] (optional) when it flushes its statistics at the end.  A separate
-// parameter struct, so that the kernels of the other modes keep their parameters and their code.
-struct RolloutPool {
-    fgp::PolicyWeights member[FG_POOL_MAX];
-    long long end[FG_POOL_MAX];
-    int count;
-    unsigned long long *stats;  // [count][4] or null
-};
-struct RolloutPoolParams : RolloutParams {
-    RolloutPool pool;
-};
-// The same with member bot_member played by the in-game BattleAI (fg_rollout_mlp_pool_bot): its CTAs run the P2 = bot
-// horizon loop, and its weight pointers are never read.
-struct RolloutPoolBotParams : RolloutPoolParams {
-    int bot_member;
-};
-
-// Observations delayed by frame_delay = depth - 1 steps (fg_rollout_mlp_delayed): the queue of every battle is the caller's
-// ring (delay_ring.cuh), advanced once per step at position (pos + t) % depth; out_* receive the delayed state after the
-// last step.  One parameter struct for every P2 mode: pool.count = 0 is no pool, bot_member = -1 no bot member.
-struct RolloutRing {
-    float4 *obs;                // [depth][n][2]
-    int32_t *frame;             // [depth][n]
-    uint32_t *misc;             // [depth][n]
-    float4 *out_obs;            // [n][2]
-    int32_t *out_frame;         // [n]
-    uint32_t *out_misc;         // [n]
-    int depth, pos;
-};
-struct RolloutDelayParams : RolloutPoolBotParams {
-    RolloutRing ring;
-};
-
-// P1 = the MLP policy, P2 = the in-game BattleAI or a second MLP policy (p2_policy), autoreset on.  Returns
-// cudaErrorInvalidValue for other hidden sizes.
+// P1 = the MLP policy, P2 = the in-game BattleAI, a second MLP policy (p2_policy) or an opponent pool, autoreset on, with
+// the frame_delay queue when ring.depth > 0.  Returns cudaErrorInvalidValue for other hidden sizes.
 cudaError_t launch_rollout(bool dense, cudaStream_t s, const RolloutParams &rp);
-// Any of the modes below or above with the frame_delay queue (P2 from rp.pool when rp.pool.count > 0).
-cudaError_t launch_rollout_delayed(bool dense, cudaStream_t s, const RolloutDelayParams &rp);
-// The same with P2 from an opponent pool (rp.p2_policy = 1; w_p2 is not read).
-cudaError_t launch_rollout_pool(bool dense, cudaStream_t s, const RolloutPoolParams &rp);
-// The same with member rp.bot_member played by the in-game bot (its weights are not read).
-cudaError_t launch_rollout_pool_bot(bool dense, cudaStream_t s, const RolloutPoolBotParams &rp);
 
 }  // namespace fgk
 #endif

@@ -1,8 +1,7 @@
 #!/usr/bin/env python3
-"""Whole-horizon rollout kernel (fg_rollout_mlp) variants: battles per lane (developer tool; the variant is chosen per
-process by FOOTSIES_B200_ROLLOUT_E).
+"""Whole-horizon rollout kernel (fg_rollout_mlp) against batch size and hidden size (developer tool).
 usage: python tools/rollout_sweep.py            # sweep
-       python tools/rollout_sweep.py --one N H  # one configuration in this process (for ncu)"""
+       python tools/rollout_sweep.py --one N H  # one configuration in this process"""
 import os
 import subprocess
 import sys
@@ -28,8 +27,7 @@ def one(n, hidden, reps=5, self_play=False, mode="horizon"):
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / reps
     fr = (env.episode_stats()["env_frames"] - f0) / reps
-    print(f"n={n} hidden={hidden} self_play={self_play} mode={mode} E={os.environ.get('FOOTSIES_B200_ROLLOUT_E', 'default')} "
-          f": {ms * 1e3 / 128:.2f} us per step, "
+    print(f"n={n} hidden={hidden} self_play={self_play} mode={mode}: {ms * 1e3 / 128:.2f} us per step, "
           f"{fr / (ms * 1e-3):.3e} env-frames/s", flush=True)
 
 
@@ -43,6 +41,4 @@ if __name__ == "__main__":
                 one(n, 64, self_play=True, mode=mode)
         sys.exit(0)
     for n, hidden in ((16384, 64), (131072, 64), (1048576, 64), (16384, 32), (16384, 128)):
-        for e in (2, 4):
-            env = dict(os.environ, FOOTSIES_B200_ROLLOUT_E=str(e))
-            subprocess.run([sys.executable, os.path.abspath(__file__), "--one", str(n), str(hidden)], env=env)
+        subprocess.run([sys.executable, os.path.abspath(__file__), "--one", str(n), str(hidden)])
